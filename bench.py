@@ -18,6 +18,14 @@ over the shard: CRC-32 check of every chunk, AES-256-CTR decrypt, zstd decode.
 `--impl reference` times the CPU path alone (the reference is Rust; there is no cargo in this image, so the oracle port runs).
 Inputs are synthetic (corpus.py), produced outside every timed region by the oracle's encoders, i.e. the same libzstd
 level-3 streaming frames / zlib level-6 streams the reference writes.
+
+`--dump-outputs DIR` writes what the last timed step of the extract and create paths returned to a caller (rank 0), so that
+two builds can be compared output for output on the same seeded inputs:
+  extract_files_sample, create_streams_sample   float32 bytes: all of them up to DUMP_SAMPLE_BYTES, beyond that windows at
+                                                 seeded places, listed as rows [entry, offset, length] in *_sample_where
+  extract_files_crc32, create_streams_crc32     float64 CRC-32 of every whole decoded file / created stream
+  extract_files_length, create_streams_length   float64 bytes of every decoded file / created stream
+  extract_chunk_crc32, create_chunk_crc32       float64 chunk CRCs the kernels computed (every chunk of the archive / FDAT)
 """
 from __future__ import annotations
 
@@ -30,6 +38,7 @@ import statistics
 import subprocess
 import sys
 import time
+import zlib
 
 import numpy as np
 
@@ -41,7 +50,39 @@ import corpus  # noqa: E402
 
 FILE_SIZE = benchlib.FILE_SIZE
 PASSWORD = b"bench-password"
+SALT = b"pna-bench-salt16"     # fixed, so that the PHSF chunks, and with them the archive bytes, repeat from run to run
 KEY = bytes(range(32))
+DUMP_SAMPLE_BYTES = 4 << 20    # per sampled output; both paths' dumps stay under 40 MB at 1024 entries
+DUMP_WINDOW = 4096
+
+
+def sample_bytes(blobs, seed: int):
+    """Bytes of `blobs` (uint8 arrays): all of them when they total at most DUMP_SAMPLE_BYTES, else windows of up to
+    DUMP_WINDOW bytes at places drawn from `seed`.  Returns (bytes as float32, rows [blob, offset, length] as float64)."""
+    lens = np.array([b.size for b in blobs], dtype=np.int64)
+    if lens.sum() <= DUMP_SAMPLE_BYTES:
+        where = np.stack([np.arange(len(blobs)), np.zeros(len(blobs), dtype=np.int64), lens], axis=1)
+    else:
+        rng = np.random.default_rng(seed)
+        k = DUMP_SAMPLE_BYTES // DUMP_WINDOW
+        blob = np.sort(rng.integers(0, len(blobs), k))
+        n = np.minimum(lens[blob], DUMP_WINDOW)
+        off = (rng.random(k) * (lens[blob] - n + 1)).astype(np.int64)
+        where = np.stack([blob, off, n], axis=1)
+    data = np.concatenate([blobs[b][o:o + n] for b, o, n in where] + [np.zeros(0, dtype=np.uint8)])
+    return data.astype(np.float32), where.astype(np.float64)
+
+
+def dump_outputs(d: str, path: str, what: str, blobs, chunk_crcs, seed: int):
+    """`path`'s outputs as DIR/<path>_<what>_{sample,sample_where,crc32,length}.npy and DIR/<path>_chunk_crc32.npy"""
+    os.makedirs(d, exist_ok=True)
+    data, where = sample_bytes(blobs, seed)
+    arrays = {f"{what}_sample": data, f"{what}_sample_where": where,
+              f"{what}_crc32": np.array([zlib.crc32(b) for b in blobs], dtype=np.float64),
+              f"{what}_length": np.array([b.size for b in blobs], dtype=np.float64),
+              "chunk_crc32": np.asarray(chunk_crcs, dtype=np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(d, f"{path}_{name}.npy"), a)
 
 
 def make_shard(rank: int, entries: int, threads: int, world: int = 1):
@@ -152,7 +193,11 @@ def main():
     ap.add_argument("--create", type=int, default=1, help="also measure the create path (GPU zstd + AES-CTR + CRC) on the same files")
     ap.add_argument("--configs", type=int, default=1, help="at N = 1: also run BASELINE.json configs 1, 3, 4, 5 at their stated sizes")
     ap.add_argument("--config-scale", type=float, default=1.0, help="shrink the configs (development runs); 1.0 = stated sizes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed extract and create steps to DIR/*.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -221,7 +266,7 @@ def main():
     plain_np, p_offs = benchlib.pack(files)
     streams_np, s_offs, _ = benchlib.oracle_encode(plain_np, p_offs, 2, 3, 1, 1, KEY, threads, seed=1234 + rank)
     Cbytes = int(s_offs[-1])
-    opts = pna.WriteOptions(compression=2, encryption=1, cipher_mode=1, password=PASSWORD, kdf_params={"i": 1000})
+    opts = pna.WriteOptions(compression=2, encryption=1, cipher_mode=1, password=PASSWORD, kdf_params={"i": 1000}, salt=SALT)
     # the shard's streams were encrypted with KEY; record it as the options' derived key (the KDF is host work, once per archive)
     archive_buf = benchlib.frame_archive(streams_np, s_offs, sizes, bytes([0, 0, 0, 2, 1, 1]), opts.phsf, 16, "corpus/%07d.bin", ctx.pinned, threads)
     arch_bytes = int(archive_buf.size)
@@ -257,6 +302,8 @@ def main():
     assert st == [0] * E and broken == 0, "decode failed"
     for k in range(0, E, max(1, E // 16)):
         assert outs[k].tobytes() == files[k], "GPU output differs from the source file"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "extract", "files", outs, crcs, seed=1)
     del outs
     plan.close()
 
@@ -334,6 +381,8 @@ def main():
             s = streams_gpu[k].tobytes()
             assert O.decode_stream(s, 2, 1, 1, KEY, None) == files[k], "GPU-created stream is not reference-readable"
             assert int(crcs_gpu[k][0]) == O.chunk_crc(b"FDAT", s[16:])
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, "create", "streams", streams_gpu, np.concatenate(crcs_gpu + [np.zeros(0, np.uint32)]), seed=2)
         eplan.close()
         ce2e = []
         names = [f"corpus/{i:07d}.bin" for i in range(E)]

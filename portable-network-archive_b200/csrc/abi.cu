@@ -287,7 +287,8 @@ struct pna_plan {
     std::vector<EntryRec> h_entries;
     std::vector<Segment> h_segs;
     std::vector<DevKeys> h_keys;
-    std::vector<CipherTile> h_tiles[5];   // 0 gather, 1 aes-ctr, 2 aes-cbc, 3 camellia-ctr, 4 camellia-cbc
+    std::vector<CipherTile> h_tiles[5];   // 0 gather, (1 unused), 2 aes-cbc, 3 camellia-ctr, 4 camellia-cbc
+    std::vector<CtrTile> h_ctr_tiles;     // aes-ctr
     std::vector<uint32_t> h_store, h_deflate, h_xz;
     // GCM STREAM (cipher mode 2): segments, 16 KiB warp tiles (AES tiles first, then Camellia), one power table per entry
     std::vector<gcm::GcmSeg> h_gcm_segs;
@@ -310,6 +311,7 @@ struct pna_plan {
     DevArr<Segment> d_segs;
     DevArr<DevKeys> d_keys;
     DevArr<CipherTile> d_tiles[5];
+    DevArr<CtrTile> d_ctr_tiles;
     DevArr<uint32_t> d_deflate, d_seq_order, d_lit_order, d_counts, d_lz_order;
     DevArr<zs::SeqRec> d_seqs;
     DevArr<zs::ZEntry> d_ze;
@@ -366,6 +368,7 @@ struct pna_plan {
         d_segs.release(); d_keys.release();
         d_gcm_segs.release(); d_gcm_tiles.release(); d_gcm_refs.release(); d_gcm_pows.release(); d_gcm_partial.release();
         for (auto& t : d_tiles) t.release();
+        d_ctr_tiles.release();
         d_deflate.release(); d_seqs.release(); d_seq_order.release(); d_lit_order.release(); d_counts.release(); d_lz_order.release(); d_lz_units.release(); d_ze.release(); d_blocks.release();
         d_lit_base.release(); d_seq_base.release(); d_copy.release();
         d_walk.release(); d_pj_segs.release(); d_pj_ptr.release(); d_pj_cpos.release(); d_pj_flags.release(); d_pj_tiles.release();
@@ -440,7 +443,7 @@ static int ctx_create_single(pna_ctx** out, int device_id) {
     delete hc;
     // opt in to the large dynamic shared memory the table-driven kernels use
     const int aes_smem = 256 * 32 * 4 + 256, cam_smem = 2 * 2048 * 4;
-    ok = ok && cudaFuncSetAttribute(decrypt_tiles_kernel<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, AES_CTR_SMEM) == cudaSuccess;
+    ok = ok && cudaFuncSetAttribute(aes_ctr_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AES_CTR_TILES_SMEM) == cudaSuccess;
     ok = ok && cudaFuncSetAttribute(decrypt_tiles_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, aes_smem) == cudaSuccess;
     ok = ok && cudaFuncSetAttribute(decrypt_tiles_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cam_smem) == cudaSuccess;
     ok = ok && cudaFuncSetAttribute(decrypt_tiles_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, cam_smem) == cudaSuccess;
@@ -651,6 +654,48 @@ static bool size_hint_trusted(uint8_t compression, uint64_t comp_len, uint64_t h
 }
 extern "C" int pna_cuda_size_hint_trusted(uint8_t compression, uint64_t stream_len, uint64_t hint) { return size_hint_trusted(compression, stream_len, hint) ? 1 : 0; }
 struct CrcReq { const pna_span* spans; const uint32_t* expect; const int32_t* entry_of; uint32_t n; const uint8_t* image; uint64_t image_len; };
+// AES-CTR tiles of entry i (aes_ctr_tiles_kernel): cut at body boundaries and after CTR_TILE_RUNS counter runs; a block that
+// straddles two bodies becomes a one-block tile gathered through the segments.  The IV is read here, from the host bodies.
+static void ctr_tiles(pna_plan* P, const pna_decode_desc& d, uint32_t i) {
+    const EntryRec& e = P->h_entries[i];
+    uint8_t ivb[16];
+    uint64_t got = 0;
+    for (uint32_t b = 0; b < d.n_bodies && got < 16; b++) {
+        const uint64_t k = std::min<uint64_t>(d.bodies[b].len, 16 - got);
+        if (k) memcpy(ivb + got, d.bodies[b].ptr, k);
+        got += k;
+    }
+    uint32_t iv[4];
+    memcpy(iv, ivb, 16);
+    const Segment* sg = P->h_segs.data() + e.seg_begin;
+    const uint64_t clen = e.comp_len, nb = (clen + 15) / 16;
+    uint32_t si = 0;
+    for (uint64_t b = 0; b < nb;) {
+        const uint64_t pos = 16 + 16 * b, rest = clen - 16 * b;
+        while (si + 1 < e.n_segs && sg[si + 1].pos <= pos) si++;
+        const uint64_t seg_end = si + 1 < e.n_segs ? sg[si + 1].pos : e.stream_len;
+        CtrTile t;
+        memset(&t, 0, sizeof t);
+        ctr128be_add(iv, b, t.ctr);
+        t.dst = e.comp_off + 16 * b;
+        t.key_idx = (uint32_t)e.key_idx;
+        t.entry = i;
+        t.pos = pos;
+        uint64_t n;
+        if (std::min<uint64_t>(rest, 16) > seg_end - pos) {   // straddles two bodies
+            t.src = CTR_TILE_SLOW;
+            n = 1;
+        } else {
+            t.src = sg[si].img_off + (pos - sg[si].pos);
+            n = rest <= seg_end - pos ? nb - b : (seg_end - pos) / 16;
+            n = std::min<uint64_t>(n, 256 * CTR_TILE_RUNS - (t.ctr[3] >> 24));
+        }
+        t.n_bytes = (uint32_t)std::min<uint64_t>(16 * n, rest);
+        P->h_ctr_tiles.push_back(t);
+        b += n;
+    }
+}
+
 static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_t n, const uint64_t* caps, const CrcReq* crc,
                              pna_plan* P) {
     P->ctx = ctx; P->kind = 0; P->n = n;
@@ -797,6 +842,10 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
             cur += align_up(e.comp_len, 16) + 16;
             const uint64_t nb = (e.comp_len + 15) / 16;
             if (e.encryption && e.cipher_mode == PNA_CIPHER_GCM) continue;   // tiled per segment below
+            if (e.encryption == PNA_ENCRYPTION_AES && e.cipher_mode == PNA_CIPHER_CTR) {
+                ctr_tiles(P, descs[i], i);
+                continue;
+            }
             std::vector<CipherTile>& tv = P->h_tiles[variant_of(e)];
             for (uint64_t b0 = 0; b0 < nb; b0 += CIPHER_TILE_BLOCKS)
                 tv.push_back({i, (uint32_t)std::min<uint64_t>(CIPHER_TILE_BLOCKS, nb - b0), b0});
@@ -866,6 +915,10 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
     if (rc) return rc;
     if (!P->h_segs.empty()) CK(cudaMemcpyAsync(P->d_segs.p, P->h_segs.data(), P->h_segs.size() * sizeof(Segment), cudaMemcpyHostToDevice, ctx->stream));
     if (!P->h_keys.empty()) CK(cudaMemcpyAsync(P->d_keys.p, P->h_keys.data(), P->h_keys.size() * sizeof(DevKeys), cudaMemcpyHostToDevice, ctx->stream));
+    if (!P->h_ctr_tiles.empty()) {
+        CK(P->d_ctr_tiles.reserve(P->h_ctr_tiles.size()));
+        CK(cudaMemcpyAsync(P->d_ctr_tiles.p, P->h_ctr_tiles.data(), P->h_ctr_tiles.size() * sizeof(CtrTile), cudaMemcpyHostToDevice, ctx->stream));
+    }
     for (int v = 0; v < 5; v++) {
         if (P->h_tiles[v].empty()) continue;
         CK(P->d_tiles[v].reserve(P->h_tiles[v].size()));
@@ -995,14 +1048,18 @@ static int launch_crc(pna_plan* P) {
 static int launch_cipher(pna_plan* P) {
     pna_ctx* ctx = P->ctx;
     const int aes_smem = 256 * 32 * 4 + 256, cam_smem = 2 * 2048 * 4;
+    if (const uint32_t nt = (uint32_t)P->h_ctr_tiles.size()) {
+        aes_ctr_tiles_kernel<<<std::min<uint32_t>(nt, (uint32_t)ctx->sm_count), AES_CTR_THREADS, AES_CTR_TILES_SMEM, ctx->stream>>>(
+            P->d_buf.p, P->d_segs.p, P->d_entries.p, P->d_ctr_tiles.p, nt, P->d_keys.p, ctx->d_aes);
+        LAUNCHED();
+    }
     for (int v = 0; v < 5; v++) {
         const uint32_t nt = (uint32_t)P->h_tiles[v].size();
         if (!nt) continue;
-        const uint32_t grid = std::min<uint32_t>(nt, (uint32_t)ctx->sm_count * (v == 1 || v == 2 ? 4 : 6));
+        const uint32_t grid = std::min<uint32_t>(nt, (uint32_t)ctx->sm_count * (v == 2 ? 4 : 6));
 #define ARGS P->d_buf.p, P->d_segs.p, P->d_entries.p, P->d_tiles[v].p, nt, P->d_keys.p, ctx->d_aes, ctx->d_cam
         switch (v) {
             case 0: decrypt_tiles_kernel<0, 1><<<grid, 256, 0, ctx->stream>>>(ARGS); break;
-            case 1: decrypt_tiles_kernel<1, 1><<<std::min<uint32_t>(nt, (uint32_t)ctx->sm_count), AES_CTR_THREADS, AES_CTR_SMEM, ctx->stream>>>(ARGS); break;
             case 2: decrypt_tiles_kernel<1, 0><<<grid, 256, aes_smem, ctx->stream>>>(ARGS); break;
             case 3: decrypt_tiles_kernel<2, 1><<<grid, 256, cam_smem, ctx->stream>>>(ARGS); break;
             case 4: decrypt_tiles_kernel<2, 0><<<grid, 256, cam_smem, ctx->stream>>>(ARGS); break;

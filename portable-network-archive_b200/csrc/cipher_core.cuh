@@ -96,27 +96,94 @@ inline void aes256_expand_key(const AesTables* T, const uint8_t key[32], AesKey*
     }
 }
 
-// s[4] in/out, rk = 60 words (any address space).  te = Te0 view, sb = (Te0>>8)&0xff gives S.
-// Same cipher with the four rotations of Te0 as four tables (Te_k[x] = rotl(Te0[x], 8k)): no rotate per lookup.  Used by the
-// CTR tile kernels, which are instruction-issue bound (16 lookups + 12 rotates + xors per round and column set).
-template <class Tab>
-PNA_HD void aes256_encrypt_block4(uint32_t s[4], const uint32_t* rk, const Tab& t0, const Tab& t1, const Tab& t2, const Tab& t3) {
-    uint32_t a = s[0] ^ rk[0], b = s[1] ^ rk[1], c = s[2] ^ rk[2], d = s[3] ^ rk[3];
+// The CTR / GCM keystream runs the cipher with the four rotations of Te0 as four tables (Te_K[x] = rotl(Te0[x], 8K)): no
+// rotate per lookup.  A four-table view T4 provides  T4::at<K, B>(v) = Te_K[byte B of v].
+// Host (and the CPU test tier): Te0 alone, rotated per lookup.
+struct Te0Rot {
+    const uint32_t* te0;
+    template <int K, int B>
+    PNA_HD uint32_t at(uint32_t v) const {
+        const uint32_t e = te0[(v >> (8 * B)) & 0xFFu];
+        return K ? rotl32(e, 8 * K) : e;
+    }
+};
+#if defined(__CUDACC__) || defined(PNA_EMU)
+// Device: the four tables replicated per lane in shared memory (128 KB), laid out [K >> 1][x][K & 1][lane].  The byte offset
+// of a lookup is  x << 8 | lane * 4  (plus the table's constant): ONE byte permute builds it from the state word, and the
+// table is picked by the load's immediate offset.  Lane l only ever reads bank l, so a warp's 32 lookups never conflict.
+constexpr uint32_t AES_TE4_WORDS = 4 * 256 * 32;
+__device__ __forceinline__ void aes_te4_fill(uint32_t* s_tab, const AesTables* aes) {
+    for (uint32_t i = threadIdx.x; i < AES_TE4_WORDS; i += blockDim.x) {
+        const uint32_t k = 2 * (i >> 14) + ((i >> 5) & 1);
+        const uint32_t e = aes->te0[(i >> 6) & 255];
+        s_tab[i] = k ? rotl32(e, 8 * k) : e;
+    }
+}
+struct LaneTe4 {
+    const uint8_t* tab;   // aes_te4_fill's tables
+    uint32_t lane4;       // lane * 4
+    template <int K, int B>
+    __device__ __forceinline__ uint32_t at(uint32_t v) const {
+        const uint32_t off = __byte_perm(v, lane4, 0x5504u | (B << 4));   // byte 0: lane4, byte 1: byte B of v, bytes 2-3: 0
+        return *reinterpret_cast<const uint32_t*>(tab + ((K >> 1) * 65536 + (K & 1) * 128) + off);
+    }
+};
+#endif
+
+// Last-round bytes: the S-box byte of Te_K[x] sits at byte (1 + K) & 3.
+PNA_HD uint32_t aes_last_bytes(uint32_t r0, uint32_t r1, uint32_t r2, uint32_t r3) {
+#if defined(__CUDA_ARCH__)
+    return __byte_perm(__byte_perm(r0, r1, 0x0061u), __byte_perm(r2, r3, 0x4300u), 0x7610u);
+#else
+    return ((r0 >> 8) & 0xFFu) | ((r1 >> 8) & 0xFF00u) | ((r2 >> 8) & 0xFF0000u) | (r3 << 24);
+#endif
+}
+
+// Rounds R0..13 and the last round on the columns a..d (which carry round key R0 - 1); rk = 60 words (any address space).
+template <int R0, class T4>
+PNA_HD void aes256_rounds4(uint32_t s[4], uint32_t a, uint32_t b, uint32_t c, uint32_t d, const uint32_t* rk, const T4& t) {
 #pragma unroll
-    for (int r = 1; r < 14; r++) {
-        const uint32_t na = t0(a & 0xFF) ^ t1((b >> 8) & 0xFF) ^ t2((c >> 16) & 0xFF) ^ t3(d >> 24) ^ rk[4 * r + 0];
-        const uint32_t nb = t0(b & 0xFF) ^ t1((c >> 8) & 0xFF) ^ t2((d >> 16) & 0xFF) ^ t3(a >> 24) ^ rk[4 * r + 1];
-        const uint32_t nc = t0(c & 0xFF) ^ t1((d >> 8) & 0xFF) ^ t2((a >> 16) & 0xFF) ^ t3(b >> 24) ^ rk[4 * r + 2];
-        const uint32_t nd = t0(d & 0xFF) ^ t1((a >> 8) & 0xFF) ^ t2((b >> 16) & 0xFF) ^ t3(c >> 24) ^ rk[4 * r + 3];
+    for (int r = R0; r < 14; r++) {
+        const uint32_t na = t.template at<0, 0>(a) ^ t.template at<1, 1>(b) ^ t.template at<2, 2>(c) ^ t.template at<3, 3>(d) ^ rk[4 * r + 0];
+        const uint32_t nb = t.template at<0, 0>(b) ^ t.template at<1, 1>(c) ^ t.template at<2, 2>(d) ^ t.template at<3, 3>(a) ^ rk[4 * r + 1];
+        const uint32_t nc = t.template at<0, 0>(c) ^ t.template at<1, 1>(d) ^ t.template at<2, 2>(a) ^ t.template at<3, 3>(b) ^ rk[4 * r + 2];
+        const uint32_t nd = t.template at<0, 0>(d) ^ t.template at<1, 1>(a) ^ t.template at<2, 2>(b) ^ t.template at<3, 3>(c) ^ rk[4 * r + 3];
         a = na; b = nb; c = nc; d = nd;
     }
-    // last round: S-box bytes.  Te0 = (2s, s, s, 3s): byte 1 of Te0[x] is s; in Te_k it sits at byte (1 + k) & 3
-#define PNA_SB0(x) ((t0(x) >> 8) & 0xFFu)
-    s[0] = (PNA_SB0(a & 0xFF) | (t1((b >> 8) & 0xFF) & 0xFF0000u) >> 8 | (t2((c >> 16) & 0xFF) & 0xFF000000u) >> 8 | (t3(d >> 24) & 0xFFu) << 24) ^ rk[56];
-    s[1] = (PNA_SB0(b & 0xFF) | (t1((c >> 8) & 0xFF) & 0xFF0000u) >> 8 | (t2((d >> 16) & 0xFF) & 0xFF000000u) >> 8 | (t3(a >> 24) & 0xFFu) << 24) ^ rk[57];
-    s[2] = (PNA_SB0(c & 0xFF) | (t1((d >> 8) & 0xFF) & 0xFF0000u) >> 8 | (t2((a >> 16) & 0xFF) & 0xFF000000u) >> 8 | (t3(b >> 24) & 0xFFu) << 24) ^ rk[58];
-    s[3] = (PNA_SB0(d & 0xFF) | (t1((a >> 8) & 0xFF) & 0xFF0000u) >> 8 | (t2((b >> 16) & 0xFF) & 0xFF000000u) >> 8 | (t3(c >> 24) & 0xFFu) << 24) ^ rk[59];
-#undef PNA_SB0
+    s[0] = aes_last_bytes(t.template at<0, 0>(a), t.template at<1, 1>(b), t.template at<2, 2>(c), t.template at<3, 3>(d)) ^ rk[56];
+    s[1] = aes_last_bytes(t.template at<0, 0>(b), t.template at<1, 1>(c), t.template at<2, 2>(d), t.template at<3, 3>(a)) ^ rk[57];
+    s[2] = aes_last_bytes(t.template at<0, 0>(c), t.template at<1, 1>(d), t.template at<2, 2>(a), t.template at<3, 3>(b)) ^ rk[58];
+    s[3] = aes_last_bytes(t.template at<0, 0>(d), t.template at<1, 1>(a), t.template at<2, 2>(b), t.template at<3, 3>(c)) ^ rk[59];
+}
+// s[4] in/out
+template <class T4>
+PNA_HD void aes256_encrypt_block4(uint32_t s[4], const uint32_t* rk, const T4& t) {
+    aes256_rounds4<1>(s, s[0] ^ rk[0], s[1] ^ rk[1], s[2] ^ rk[2], s[3] ^ rk[3], rk, t);
+}
+
+// AES-256-CTR over a counter run: up to 256 consecutive counter blocks that share bytes 0..14 (only the low byte x, byte 15,
+// counts).  Byte 15 is byte 3 of column d, so in round 1 it reaches one lookup (column a's Te3) and in round 2 it reaches,
+// through round-1 column a, one lookup per column.  aes256_ctr_run_init computes once per run everything else of rounds 1-2
+// (27 lookups): p[0] = round-1 column a without its Te3 term, p[1..4] = round-2 columns a..d without their term in round-1
+// column a.  aes256_ctr_run_block then encrypts the run's block x with 5 lookups for rounds 1-2 instead of 32.
+template <class T4>
+PNA_HD void aes256_ctr_run_init(const uint32_t ctr[4], const uint32_t* rk, const T4& t, uint32_t p[5]) {
+    const uint32_t a = ctr[0] ^ rk[0], b = ctr[1] ^ rk[1], c = ctr[2] ^ rk[2], d = ctr[3] ^ rk[3];
+    p[0] = t.template at<0, 0>(a) ^ t.template at<1, 1>(b) ^ t.template at<2, 2>(c) ^ rk[4];
+    const uint32_t b1 = t.template at<0, 0>(b) ^ t.template at<1, 1>(c) ^ t.template at<2, 2>(d) ^ t.template at<3, 3>(a) ^ rk[5];
+    const uint32_t c1 = t.template at<0, 0>(c) ^ t.template at<1, 1>(d) ^ t.template at<2, 2>(a) ^ t.template at<3, 3>(b) ^ rk[6];
+    const uint32_t d1 = t.template at<0, 0>(d) ^ t.template at<1, 1>(a) ^ t.template at<2, 2>(b) ^ t.template at<3, 3>(c) ^ rk[7];
+    p[1] = t.template at<1, 1>(b1) ^ t.template at<2, 2>(c1) ^ t.template at<3, 3>(d1) ^ rk[8];    // lacks Te0[a1 byte 0]
+    p[2] = t.template at<0, 0>(b1) ^ t.template at<1, 1>(c1) ^ t.template at<2, 2>(d1) ^ rk[9];    // lacks Te3[a1 byte 3]
+    p[3] = t.template at<0, 0>(c1) ^ t.template at<1, 1>(d1) ^ t.template at<3, 3>(b1) ^ rk[10];   // lacks Te2[a1 byte 2]
+    p[4] = t.template at<0, 0>(d1) ^ t.template at<2, 2>(b1) ^ t.template at<3, 3>(c1) ^ rk[11];   // lacks Te1[a1 byte 1]
+}
+// x24 = the block's counter low byte in bits 24..31 (other bits zero); s = E_K(counter)
+template <class T4>
+PNA_HD void aes256_ctr_run_block(const uint32_t p[5], uint32_t x24, const uint32_t* rk, const T4& t, uint32_t s[4]) {
+    const uint32_t a1 = p[0] ^ t.template at<3, 3>(x24 ^ rk[3]);
+    aes256_rounds4<3>(s, p[1] ^ t.template at<0, 0>(a1), p[2] ^ t.template at<3, 3>(a1), p[3] ^ t.template at<2, 2>(a1),
+                      p[4] ^ t.template at<1, 1>(a1), rk, t);
 }
 
 template <class Tab>

@@ -224,25 +224,19 @@ struct DevKeys {   // one per distinct (cipher, key)
 };
 
 // dynamic shared memory layout: [AES table 256*32 u32 (replicated)] or [Camellia sp_hi|sp_lo 2*2048 u32],
-// then per-CTA key words.
-// AES-CTR (ENC 1, MODE 1) runs 1024 threads per CTA over FOUR replicated tables (128 KB of shared memory, one CTA per SM);
-// every other variant 256 threads over one table.
-constexpr int AES_CTR_THREADS = 1024;
-constexpr int AES_CTR_SMEM = 4 * 256 * 32 * 4 + 256;
+// then per-CTA key words.  256 threads per CTA.  AES-CTR has its own kernel (aes_ctr_tiles_kernel).
 template <int ENC /*1 aes, 2 camellia, 0 none*/, int MODE /*0 cbc, 1 ctr*/>
-__global__ void __launch_bounds__(ENC == 1 && MODE == 1 ? AES_CTR_THREADS : 256) decrypt_tiles_kernel(uint8_t* __restrict__ buf, const Segment* __restrict__ segs,
+__global__ void __launch_bounds__(256) decrypt_tiles_kernel(uint8_t* __restrict__ buf, const Segment* __restrict__ segs,
                                                             EntryRec* __restrict__ entries,
                                                             const CipherTile* __restrict__ tiles, uint32_t n_tiles,
                                                             const DevKeys* __restrict__ keys,
                                                             const AesTables* __restrict__ aes,
                                                             const CamelliaTables* __restrict__ cam) {
+    static_assert(!(ENC == 1 && MODE == 1), "AES-CTR runs aes_ctr_tiles_kernel");
     extern __shared__ uint32_t smem[];
     uint32_t* s_tab = smem;
     uint8_t* s_isb = nullptr;
-    if (ENC == 1 && MODE == 1) {
-        for (int i = threadIdx.x; i < 4 * 256 * 32; i += blockDim.x)                       // [k][x*32 + lane] = rotl(Te0[x], 8k)
-            s_tab[i] = rotl32(aes->te0[(i >> 5) & 255], 8 * (i >> 13));
-    } else if (ENC == 1) {
+    if (ENC == 1) {
         const uint32_t* src = aes->td0;
         for (int i = threadIdx.x; i < 256 * 32; i += blockDim.x) s_tab[i] = src[i >> 5];   // [x*32 + lane]
         s_isb = reinterpret_cast<uint8_t*>(smem + 256 * 32);
@@ -267,7 +261,7 @@ __global__ void __launch_bounds__(ENC == 1 && MODE == 1 ? AES_CTR_THREADS : 256)
         if (ENC != 0 && e.key_idx != s_key_idx) {   // (re)load round keys for this tile's entry
             __syncthreads();
             const DevKeys* k = keys + e.key_idx;
-            if (ENC == 1) { if (threadIdx.x < 60) s_key32[threadIdx.x] = MODE == 1 ? k->aes_rk[threadIdx.x] : k->aes_dk[threadIdx.x]; }
+            if (ENC == 1) { if (threadIdx.x < 60) s_key32[threadIdx.x] = k->aes_dk[threadIdx.x]; }
             else { if (threadIdx.x < 34) s_key64[threadIdx.x] = MODE == 1 ? k->cam_ek[threadIdx.x] : k->cam_dk[threadIdx.x]; }
             if (threadIdx.x == 0) s_key_idx = e.key_idx;
             __syncthreads();
@@ -288,10 +282,7 @@ __global__ void __launch_bounds__(ENC == 1 && MODE == 1 ? AES_CTR_THREADS : 256)
             if (ENC == 0) { o[0] = c[0]; o[1] = c[1]; o[2] = c[2]; o[3] = c[3]; }
             else if (MODE == 1) {   // CTR: keystream = E(IV + bi)
                 ctr128be_add(iv, bi, o);
-                if (ENC == 1) {
-                    const TabView t1{s_tab + 8192, 32, tv.lane}, t2{s_tab + 16384, 32, tv.lane}, t3{s_tab + 24576, 32, tv.lane};
-                    aes256_encrypt_block4(o, s_key32, tv, t1, t2, t3);
-                } else camellia256_crypt_block(o, s_key64, s_tab, s_tab + 2048);
+                camellia256_crypt_block(o, s_key64, s_tab, s_tab + 2048);
                 o[0] ^= c[0]; o[1] ^= c[1]; o[2] ^= c[2]; o[3] ^= c[3];
             } else {                // CBC: P = D(C_i) ^ C_{i-1}
                 uint32_t prev[4];
@@ -312,6 +303,116 @@ __global__ void __launch_bounds__(ENC == 1 && MODE == 1 ? AES_CTR_THREADS : 256)
             }
             if (have == 16) *reinterpret_cast<uint4*>(dst + bi * 16) = make_uint4(o[0], o[1], o[2], o[3]);
             else for (uint32_t k = 0; k < have; k++) dst[bi * 16 + k] = (uint8_t)(o[k >> 2] >> (8 * (k & 3)));
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// AES-256-CTR extract.  A tile is a contiguous piece of ONE body (the host cuts tiles at body boundaries) and carries what a
+// block would otherwise look up: its image offset, its destination and the counter block of its first block.  A tile spans
+// at most CTR_TILE_RUNS counter runs (aes256_ctr_run_init), one per warp: lane l of warp w takes the blocks of run w whose
+// counter low byte is l, l + 32, .., l + 224 -- up to 8 blocks that share the run's rounds 1-2, contiguous across the warp so
+// that loads and stores coalesce.  A block that straddles two bodies is a tile of its own (src == CTR_TILE_SLOW), gathered
+// through the entry's segments.
+struct CtrTile {
+    uint64_t src;       // image offset of the first ciphertext byte, or CTR_TILE_SLOW
+    uint64_t dst;       // arena offset of the first output byte (16-byte aligned)
+    uint32_t ctr[4];    // counter block of the first block (IV + block index), words as loaded
+    uint32_t n_bytes;   // ciphertext bytes (the entry's last block may be partial)
+    uint32_t key_idx;
+    uint32_t entry;     // CTR_TILE_SLOW: whose segments to gather from ...
+    uint32_t _pad;
+    uint64_t pos;       // ... starting at this stream position
+};
+constexpr uint64_t CTR_TILE_SLOW = ~(uint64_t)0;
+constexpr uint32_t CTR_TILE_RUNS = 32;                 // = warps per CTA
+constexpr int AES_CTR_THREADS = 1024;                  // one CTA per SM: the tables take 128 KB
+constexpr int AES_CTR_SMEM = AES_TE4_WORDS * 4 + 256;  // the create kernel keeps its keys in static shared memory
+constexpr int AES_CTR_TILES_SMEM = AES_TE4_WORDS * 4 + CTR_TILE_RUNS * 64 * 4;   // + each warp's round keys
+// n <= 16 stream bytes at stream position pos of entry *e, any segmentation (kept out of the kernel's hot loop)
+__device__ __noinline__ uint4 ctr_gather_block(const uint8_t* buf, const Segment* segs, const EntryRec* e, uint64_t pos, uint32_t n) {
+    uint32_t w[4] = {0, 0, 0, 0};
+    if (n == 16) { load_stream16(buf, segs + e->seg_begin, e->n_segs, e->stream_len, pos, w); return make_uint4(w[0], w[1], w[2], w[3]); }
+    uint64_t lo = 0, hi = 0;   // no register array indexed at run time: it would go to local memory
+    for (uint32_t k = 0; k < n; k++) {
+        const uint64_t v = load_stream1(buf, segs + e->seg_begin, e->n_segs, pos + k);
+        if (k < 8) lo |= v << (8 * k); else hi |= v << (8 * (k - 8));
+    }
+    return make_uint4((uint32_t)lo, (uint32_t)(lo >> 32), (uint32_t)hi, (uint32_t)(hi >> 32));
+}
+__global__ void __launch_bounds__(AES_CTR_THREADS, 1) aes_ctr_tiles_kernel(uint8_t* __restrict__ buf, const Segment* __restrict__ segs,
+                                                                           const EntryRec* __restrict__ entries,
+                                                                           const CtrTile* __restrict__ tiles, uint32_t n_tiles,
+                                                                           const DevKeys* __restrict__ keys,
+                                                                           const AesTables* __restrict__ aes) {
+    extern __shared__ __align__(16) uint32_t smem[];
+    aes_te4_fill(smem, aes);
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t* const s_rk = smem + AES_TE4_WORDS + 64 * warp;
+    __syncthreads();
+    const LaneTe4 t{reinterpret_cast<const uint8_t*>(smem), lane * 4};
+    const uint32_t* const rk = static_cast<const uint32_t*>(__builtin_assume_aligned(s_rk, 16));
+    uint32_t have_key = 0xFFFFFFFFu;
+    for (uint32_t ti = blockIdx.x; ti < n_tiles; ti += gridDim.x) {
+        const CtrTile tl = tiles[ti];
+        const uint32_t n_blocks = (tl.n_bytes + 15) / 16;
+        const int32_t j0 = (int32_t)(256 * warp) - (int32_t)(tl.ctr[3] >> 24);   // tile block of this run's low byte 0
+        if (j0 + 256 <= 0 || j0 >= (int32_t)n_blocks) continue;                  // the tile has no block in run `warp`
+        if (tl.key_idx != have_key) {
+            __syncwarp();
+            for (uint32_t i = lane; i < 60; i += 32) s_rk[i] = keys[tl.key_idx].aes_rk[i];
+            have_key = tl.key_idx;
+            __syncwarp();
+        }
+        uint32_t run[4] = {tl.ctr[0], tl.ctr[1], tl.ctr[2], tl.ctr[3] & 0x00FFFFFFu};
+        ctr128be_add(run, 256u * warp, run);   // carries through all 128 bits and wraps at 2^128
+        uint32_t p[5];
+        aes256_ctr_run_init(run, rk, t, p);
+
+        const bool slow = tl.src == CTR_TILE_SLOW;
+        const uintptr_t sa = reinterpret_cast<uintptr_t>(buf) + (slow ? 0 : tl.src);
+        const uint4* const q = reinterpret_cast<const uint4*>(sa & ~(uintptr_t)15);   // aligned 16-byte words of the tile
+        const uint32_t wo = (uint32_t)(sa >> 2) & 3, sh = (uint32_t)(sa & 3) * 8;
+        // ciphertext of tile block j: the enclosing aligned 16 bytes and the next, then a funnel shift (bodies are not aligned)
+        auto load = [&](int32_t j, uint32_t c[4]) {
+            if (slow) {
+                const uint4 v = ctr_gather_block(buf, segs, entries + tl.entry, tl.pos, tl.n_bytes);
+                c[0] = v.x; c[1] = v.y; c[2] = v.z; c[3] = v.w;
+                return;
+            }
+            const uint4 a = __ldg(q + j);
+            const uint4 b = (sa & 15) ? __ldg(q + j + 1) : make_uint4(0, 0, 0, 0);
+            uint32_t v0, v1, v2, v3, v4;
+            switch (wo) {
+                case 0: v0 = a.x; v1 = a.y; v2 = a.z; v3 = a.w; v4 = b.x; break;
+                case 1: v0 = a.y; v1 = a.z; v2 = a.w; v3 = b.x; v4 = b.y; break;
+                case 2: v0 = a.z; v1 = a.w; v2 = b.x; v3 = b.y; v4 = b.z; break;
+                default: v0 = a.w; v1 = b.x; v2 = b.y; v3 = b.z; v4 = b.w; break;
+            }
+            c[0] = __funnelshift_r(v0, v1, sh); c[1] = __funnelshift_r(v1, v2, sh);
+            c[2] = __funnelshift_r(v2, v3, sh); c[3] = __funnelshift_r(v3, v4, sh);
+        };
+        auto in_tile = [&](int32_t j) { return j >= 0 && j < (int32_t)n_blocks; };
+        uint8_t* const dst = buf + tl.dst;
+        uint32_t c[4] = {0, 0, 0, 0};
+        if (in_tile(j0 + (int32_t)lane)) load(j0 + (int32_t)lane, c);
+#pragma unroll 1
+        for (uint32_t x = lane; x < 256; x += 32) {
+            const int32_t j = j0 + (int32_t)x;
+            uint32_t cn[4] = {0, 0, 0, 0};
+            if (x + 32 < 256 && in_tile(j + 32)) load(j + 32, cn);   // the keystream does not wait for the data
+            if (in_tile(j)) {
+                uint32_t o[4];
+                aes256_ctr_run_block(p, x << 24, rk, t, o);
+                o[0] ^= c[0]; o[1] ^= c[1]; o[2] ^= c[2]; o[3] ^= c[3];
+                const uint32_t have = tl.n_bytes - 16 * (uint32_t)j;
+                if (have >= 16) *reinterpret_cast<uint4*>(dst + 16 * (uint32_t)j) = make_uint4(o[0], o[1], o[2], o[3]);
+                else {
+                    const uint64_t lo = o[0] | (uint64_t)o[1] << 32, hi = o[2] | (uint64_t)o[3] << 32;
+                    for (uint32_t k = 0; k < have; k++) dst[16 * (uint32_t)j + k] = (uint8_t)(k < 8 ? lo >> (8 * k) : hi >> (8 * (k - 8)));
+                }
+            }
+            c[0] = cn[0]; c[1] = cn[1]; c[2] = cn[2]; c[3] = cn[3];
         }
     }
 }

@@ -457,9 +457,7 @@ __global__ void __launch_bounds__(ENC == 1 ? AES_CTR_THREADS : 256) encrypt_tile
                                                             const CamelliaTables* __restrict__ cam, uint8_t* __restrict__ out) {
     extern __shared__ uint32_t smem[];
     uint32_t* s_tab = smem;
-    if (ENC == 1) {   // four replicated tables [k][x*32 + lane] = rotl(Te0[x], 8k), 1024 threads per CTA (see decrypt_tiles_kernel)
-        for (int i = threadIdx.x; i < 4 * 256 * 32; i += blockDim.x) s_tab[i] = rotl32(aes->te0[(i >> 5) & 255], 8 * (i >> 13));
-    }
+    if (ENC == 1) aes_te4_fill(s_tab, aes);   // four lane-replicated tables, 1024 threads per CTA (see aes_ctr_tiles_kernel)
     else if (ENC == 2) {
         for (int i = threadIdx.x; i < 2048; i += blockDim.x) { s_tab[i] = (&cam->sp_hi[0][0])[i]; s_tab[2048 + i] = (&cam->sp_lo[0][0])[i]; }
     }
@@ -468,7 +466,6 @@ __global__ void __launch_bounds__(ENC == 1 ? AES_CTR_THREADS : 256) encrypt_tile
     __shared__ int s_key_idx;
     if (threadIdx.x == 0) s_key_idx = -2;
     __syncthreads();
-    const TabView tv{s_tab, 32, (uint32_t)(threadIdx.x & 31)};
     for (uint32_t t = blockIdx.x; t < n_tiles; t += gridDim.x) {
         const CipherTile tl = tiles[t];
         const EncEntry& e = entries[tl.entry];
@@ -499,10 +496,7 @@ __global__ void __launch_bounds__(ENC == 1 ? AES_CTR_THREADS : 256) encrypt_tile
             uint32_t o[4] = {c[0], c[1], c[2], c[3]};
             if (ENC != 0) {
                 ctr128be_add(iv, bi, o);
-                if (ENC == 1) {
-                    const TabView t1{s_tab + 8192, 32, tv.lane}, t2{s_tab + 16384, 32, tv.lane}, t3{s_tab + 24576, 32, tv.lane};
-                    aes256_encrypt_block4(o, s_key32, tv, t1, t2, t3);
-                }
+                if (ENC == 1) aes256_encrypt_block4(o, s_key32, LaneTe4{reinterpret_cast<const uint8_t*>(s_tab), (threadIdx.x & 31) * 4});
                 else camellia256_crypt_block(o, s_key64, s_tab, s_tab + 2048);
                 o[0] ^= c[0]; o[1] ^= c[1]; o[2] ^= c[2]; o[3] ^= c[3];
             }

@@ -94,13 +94,12 @@ __global__ void __launch_bounds__(gcm_tile_warps<ENC>() * 32) gcm_tiles_kernel(c
     constexpr int GCM_TILE_WARPS = ENC == 1 ? 32 : 8;
     GcmWarpState* ws_all = reinterpret_cast<GcmWarpState*>(smem + TAB_WORDS);
     uint32_t* s_last4 = reinterpret_cast<uint32_t*>(ws_all + GCM_TILE_WARPS);
-    if (ENC == 1) { for (int i = threadIdx.x; i < 4 * 256 * 32; i += blockDim.x) s_tab[i] = rotl32(aes->te0[(i >> 5) & 255], 8 * (i >> 13)); }   // [k][x*32 + lane]
+    if (ENC == 1) aes_te4_fill(s_tab, aes);
     else for (int i = threadIdx.x; i < 2048; i += blockDim.x) { s_tab[i] = (&cam->sp_hi[0][0])[i]; s_tab[2048 + i] = (&cam->sp_lo[0][0])[i]; }
     if (threadIdx.x < 16) { const uint32_t l4[16] = PNA_GCM_LAST4; s_last4[threadIdx.x] = l4[threadIdx.x]; }
     __syncthreads();
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     GcmWarpState& ws = ws_all[warp];
-    const TabView tv{s_tab, 32, lane};
     uint32_t have_pow = 0xFFFFFFFFu;
     const uint32_t n_warps = gridDim.x * GCM_TILE_WARPS;
     for (uint32_t t = blockIdx.x * GCM_TILE_WARPS + warp; t < n_tiles; t += n_warps) {
@@ -140,8 +139,7 @@ __global__ void __launch_bounds__(gcm_tile_warps<ENC>() * 32) gcm_tiles_kernel(c
             }
             uint32_t o[4] = {sg.nonce[0], sg.nonce[1], sg.nonce[2], bswap32((uint32_t)bi + 2u)};   // inc32 from J0 + 1
             if (ENC == 1) {
-                const TabView t1{s_tab + 8192, 32, lane}, t2{s_tab + 16384, 32, lane}, t3{s_tab + 24576, 32, lane};
-                aes256_encrypt_block4(o, ws.rk32, tv, t1, t2, t3);
+                aes256_encrypt_block4(o, ws.rk32, LaneTe4{reinterpret_cast<const uint8_t*>(s_tab), lane * 4});
             } else camellia256_crypt_block(o, ws.rk64, s_tab, s_tab + 2048);
             o[0] ^= c[0]; o[1] ^= c[1]; o[2] ^= c[2]; o[3] ^= c[3];
             if (!DECRYPT && have < 16) {   // the hash sees the ciphertext zero-padded

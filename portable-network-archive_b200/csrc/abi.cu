@@ -161,6 +161,13 @@ struct DevArr {   // growable device array (never shrinks); returned to the cach
         if (e == cudaSuccess) { p = (T*)q; cap = std::max<size_t>(n, 1); }
         return e;
     }
+    // room for n elements and their copy from the host queued on s; nothing at all (no allocation either) for n == 0
+    cudaError_t upload(const T* h, size_t n, cudaStream_t s) {
+        if (!n) return cudaSuccess;
+        const cudaError_t e = reserve(n);
+        return e == cudaSuccess ? cudaMemcpyAsync(p, h, n * sizeof(T), cudaMemcpyHostToDevice, s) : e;
+    }
+    cudaError_t upload(const std::vector<T>& h, cudaStream_t s) { return upload(h.data(), h.size(), s); }
     void release() { if (p) g_dev_cache.release(p); p = nullptr; cap = 0; }
     ~DevArr() { release(); }
     DevArr() = default;
@@ -169,6 +176,24 @@ struct DevArr {   // growable device array (never shrinks); returned to the cach
 };
 
 static inline uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
+
+// A table-driven block-cipher kernel and the dynamic shared memory it is opted in to (ctx_create_single, enc::init_attributes;
+// a kernel without any keeps the default) and launched with.  AES: Te0 or Td0 replicated per lane (32 KB), plus the inverse
+// S-box (256 bytes) where the kernel may decrypt; Camellia: sp_hi | sp_lo (16 KB).
+template <class F>
+struct CipherKernel {
+    F fn;
+    int smem;
+    bool opt_in() const { return !smem || cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess; }
+};
+constexpr int AES_SMEM = 256 * 32 * 4, AES_DEC_SMEM = AES_SMEM + 256, CAM_SMEM = 2 * 2048 * 4;
+// decode cipher-tile slots (variant_of), in launch order; AES-CTR runs aes_ctr_tiles_kernel
+static const CipherKernel<decltype(&decrypt_tiles_kernel<0, 1>)> DECRYPT_TILES[4] = {
+    {decrypt_tiles_kernel<0, 1>, 0},              // gather of plain multi-body streams
+    {decrypt_tiles_kernel<1, 0>, AES_DEC_SMEM},   // AES-CBC
+    {decrypt_tiles_kernel<2, 1>, CAM_SMEM},       // Camellia-CTR
+    {decrypt_tiles_kernel<2, 0>, CAM_SMEM}};      // Camellia-CBC
+constexpr int ECB_SMEM = AES_DEC_SMEM;
 
 namespace pna { namespace multi {
 // LPT: heaviest entries first onto the least loaded device; each device keeps its entries in caller order
@@ -273,6 +298,17 @@ struct Stager {
 constexpr int PNA_N_STAGES = 9;
 static const char* const PNA_STAGE_NAMES[PNA_N_STAGES] = {"crc", "cipher", "zstd_scan", "zstd_seq", "zstd_lit", "zstd_prefix", "zstd_lz", "inflate", "store"};
 
+// GCM STREAM (cipher mode 2) tables of a plan on the device: segments, 16 KiB warp tiles (the first n_tiles_aes of them AES,
+// the rest Camellia) with a partial GHASH each, and one key reference and power table per entry
+struct GcmDev {
+    DevArr<gcm::GcmSeg> segs;
+    DevArr<gcm::GcmTile> tiles;
+    DevArr<gcm::GcmKeyRef> refs;
+    DevArr<gcm::GcmPow> pows;
+    DevArr<gcm::G128> partial;
+    uint32_t n_segs = 0, n_tiles = 0, n_tiles_aes = 0, n_keys = 0;
+};
+
 namespace pna { namespace multi { struct Plan; } }
 // ------------------------------------------------------------------------------------------------
 struct pna_plan {
@@ -287,19 +323,14 @@ struct pna_plan {
     std::vector<EntryRec> h_entries;
     std::vector<Segment> h_segs;
     std::vector<DevKeys> h_keys;
-    std::vector<CipherTile> h_tiles[5];   // 0 gather, (1 unused), 2 aes-cbc, 3 camellia-ctr, 4 camellia-cbc
+    std::vector<CipherTile> h_tiles[4];   // by variant_of: 0 gather, 1 aes-cbc, 2 camellia-ctr, 3 camellia-cbc
     std::vector<CtrTile> h_ctr_tiles;     // aes-ctr
     std::vector<uint32_t> h_store, h_deflate, h_xz;
-    // GCM STREAM (cipher mode 2): segments, 16 KiB warp tiles (AES tiles first, then Camellia), one power table per entry
+    // GCM STREAM (cipher mode 2): the host side of `gcm`
     std::vector<gcm::GcmSeg> h_gcm_segs;
     std::vector<gcm::GcmTile> h_gcm_tiles;
     std::vector<gcm::GcmKeyRef> h_gcm_refs;
-    uint32_t n_gcm_tiles_aes = 0;
-    DevArr<gcm::GcmSeg> d_gcm_segs;
-    DevArr<gcm::GcmTile> d_gcm_tiles;
-    DevArr<gcm::GcmKeyRef> d_gcm_refs;
-    DevArr<gcm::GcmPow> d_gcm_pows;
-    DevArr<gcm::G128> d_gcm_partial;
+    GcmDev gcm;
     std::vector<inf::InfStream> h_inf;          // deflate streams of the two-stage path (tokens -> LZ -> Adler)
     std::vector<uint32_t> h_deflate_big;        // streams of 2 GiB and more: one-thread-per-stream kernel
     std::vector<zs::ZEntry> h_ze;
@@ -310,7 +341,7 @@ struct pna_plan {
     DevArr<EntryRec> d_entries, d_entries_init;
     DevArr<Segment> d_segs;
     DevArr<DevKeys> d_keys;
-    DevArr<CipherTile> d_tiles[5];
+    DevArr<CipherTile> d_tiles[4];
     DevArr<CtrTile> d_ctr_tiles;
     DevArr<uint32_t> d_deflate, d_seq_order, d_lit_order, d_counts, d_lz_order;
     DevArr<zs::SeqRec> d_seqs;
@@ -364,15 +395,6 @@ struct pna_plan {
     enc::EncodePlan* enc = nullptr;
     ~pna_plan() {
         if (ev_ready) for (auto& e : ev) { if (ctx) ctx->ev_pool.push_back(e); else cudaEventDestroy(e); }
-        d_buf.release(); d_out.release(); d_lits.release(); d_entries.release(); d_entries_init.release();
-        d_segs.release(); d_keys.release();
-        d_gcm_segs.release(); d_gcm_tiles.release(); d_gcm_refs.release(); d_gcm_pows.release(); d_gcm_partial.release();
-        for (auto& t : d_tiles) t.release();
-        d_ctr_tiles.release();
-        d_deflate.release(); d_seqs.release(); d_seq_order.release(); d_lit_order.release(); d_counts.release(); d_lz_order.release(); d_lz_units.release(); d_ze.release(); d_blocks.release();
-        d_lit_base.release(); d_seq_base.release(); d_copy.release();
-        d_walk.release(); d_pj_segs.release(); d_pj_ptr.release(); d_pj_cpos.release(); d_pj_flags.release(); d_pj_tiles.release();
-        d_inf.release(); d_inf_lits.release(); d_inf_recs.release(); d_inf_blocks.release(); d_inf_ze.release(); d_inf_tr.release(); d_xz.release(); d_xz_map.release(); d_xz_win_begin.release(); d_xz_wins.release();
         if (enc) enc::destroy(enc);
     }
 };
@@ -442,12 +464,9 @@ static int ctx_create_single(pna_ctx** out, int device_id) {
               cudaMemcpy(ctx->d_cam, &ctx->h_cam, sizeof(CamelliaTables), cudaMemcpyHostToDevice) == cudaSuccess;
     delete hc;
     // opt in to the large dynamic shared memory the table-driven kernels use
-    const int aes_smem = 256 * 32 * 4 + 256, cam_smem = 2 * 2048 * 4;
     ok = ok && cudaFuncSetAttribute(aes_ctr_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AES_CTR_TILES_SMEM) == cudaSuccess;
-    ok = ok && cudaFuncSetAttribute(decrypt_tiles_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, aes_smem) == cudaSuccess;
-    ok = ok && cudaFuncSetAttribute(decrypt_tiles_kernel<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, cam_smem) == cudaSuccess;
-    ok = ok && cudaFuncSetAttribute(decrypt_tiles_kernel<2, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, cam_smem) == cudaSuccess;
-    ok = ok && cudaFuncSetAttribute(ecb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, aes_smem) == cudaSuccess;
+    for (const auto& k : DECRYPT_TILES) ok = ok && k.opt_in();
+    ok = ok && cudaFuncSetAttribute(ecb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ECB_SMEM) == cudaSuccess;
     ok = ok && cudaFuncSetAttribute(gcm::gcm_tiles_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, gcm::gcm_tiles_smem<1>()) == cudaSuccess;
     ok = ok && cudaFuncSetAttribute(gcm::gcm_tiles_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, gcm::gcm_tiles_smem<2>()) == cudaSuccess;
     ok = ok && cudaFuncSetAttribute(gcm::gcm_tiles_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, gcm::gcm_tiles_smem<1>()) == cudaSuccess;
@@ -544,12 +563,21 @@ extern "C" int pna_cuda_transfer_probe(pna_ctx* ctx, const uint8_t* h2d_src, uin
     if (rc == PNA_OK) { cudaEventElapsedTime(&t, e[0], e[1]); if (both_ms) *both_ms = t; }
     for (auto& x : e) cudaEventDestroy(x);
     cudaStreamDestroy(s2);
-    d_in.release(); d_out.release();
     return rc;
 }
 
 // ------------------------------------------------------------------------------------------------
 // seam 1: CRC
+// CRC-32 of n spans of img, each cut into CRC_TILE tiles (first[i]: the first tile of span i): raw CRCs of the tiles, then
+// one fold per span, which starts from `init` (the register after a prefix the CRC covers but the image does not hold)
+static int launch_chunk_crc(pna_ctx* ctx, const uint8_t* img, const CrcTile* tiles, uint32_t nt, uint32_t* raw, const uint32_t* first,
+                            uint32_t n, uint32_t* crc, uint32_t init = 0xFFFFFFFFu) {
+    launch_crc_tiles(ctx->stream, ctx->sm_count, img, tiles, nt, ctx->d_crc, raw);
+    LAUNCHED();
+    crc_combine_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(tiles, raw, first, n, nt, ctx->d_crc, crc, init);
+    LAUNCHED();
+    return PNA_OK;
+}
 static int crc_run(pna_ctx* ctx, const uint8_t* d_img, const std::vector<uint64_t>& off, const uint64_t* len, uint32_t n,
                    uint32_t* crc_out) {
     std::vector<CrcTile> tiles;
@@ -566,26 +594,13 @@ static int crc_run(pna_ctx* ctx, const uint8_t* d_img, const std::vector<uint64_
     }
     const uint32_t nt = (uint32_t)tiles.size();
     DevArr<CrcTile> d_tiles; DevArr<uint32_t> d_first, d_raw, d_crc;
-    CK(d_tiles.reserve(nt)); CK(d_first.reserve(n)); CK(d_raw.reserve(nt)); CK(d_crc.reserve(n));
-    int rc = PNA_OK;
-    do {
-        cudaError_t e;
-        if ((e = cudaMemcpyAsync(d_tiles.p, tiles.data(), nt * sizeof(CrcTile), cudaMemcpyHostToDevice, ctx->stream)) != cudaSuccess ||
-            (e = cudaMemcpyAsync(d_first.p, first.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream)) != cudaSuccess) {
-            ctx->fail("crc upload", e); rc = PNA_E_CUDA; break;
-        }
-        launch_crc_tiles(ctx->stream, ctx->sm_count, d_img, d_tiles.p, nt, ctx->d_crc, d_raw.p);
-        ctx->launches++;
-        crc_combine_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(d_tiles.p, d_raw.p, d_first.p, n, nt, ctx->d_crc, d_crc.p);
-        ctx->launches++;
-        if ((e = cudaGetLastError()) != cudaSuccess ||
-            (e = cudaMemcpyAsync(crc_out, d_crc.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream)) != cudaSuccess ||
-            (e = ctx->sync()) != cudaSuccess) {
-            ctx->fail("crc run", e); rc = PNA_E_CUDA; break;
-        }
-    } while (0);
-    d_tiles.release(); d_first.release(); d_raw.release(); d_crc.release();
-    return rc;
+    CK(d_tiles.upload(tiles, ctx->stream)); CK(d_first.upload(first, ctx->stream));
+    CK(d_raw.reserve(nt)); CK(d_crc.reserve(n));
+    const int rc = launch_chunk_crc(ctx, d_img, d_tiles.p, nt, d_raw.p, d_first.p, n, d_crc.p);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(crc_out, d_crc.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx->sync());
+    return PNA_OK;
 }
 
 extern "C" int pna_cuda_crc32(pna_ctx* ctx, const pna_span* spans, uint32_t n, uint32_t* crc_out) {
@@ -602,7 +617,6 @@ extern "C" int pna_cuda_crc32(pna_ctx* ctx, const pna_span* spans, uint32_t n, u
     int rc = st.upload(ctx, d_img.p);
     if (rc == PNA_OK) rc = crc_run(ctx, d_img.p, off, len.data(), n, crc_out);
     ctx->sync();
-    d_img.release();
     return rc;
 }
 
@@ -627,15 +641,15 @@ extern "C" int pna_cuda_crc32_image(pna_ctx* ctx, const uint8_t* image, uint64_t
     std::vector<uint64_t> off(span_off, span_off + n);
     if (rc == PNA_OK) rc = crc_run(ctx, d_img.p, off, span_len, n, crc_out);
     ctx->sync();
-    d_img.release();
     return rc;
 }
 
 // ------------------------------------------------------------------------------------------------
 // seam 2: decode
+// cipher-tile slot (DECRYPT_TILES) of an entry that is neither AES-CTR nor GCM
 static int variant_of(const EntryRec& e) {
     if (e.encryption == 0) return 0;
-    return (e.encryption == 1 ? 1 : 3) + (e.cipher_mode == 1 ? 0 : 1);
+    return e.encryption == PNA_ENCRYPTION_AES ? 1 : e.cipher_mode == PNA_CIPHER_CTR ? 2 : 3;
 }
 
 // Upper bound of what a compressed stream of `comp_len` bytes can decode to: zstd emits at most one 128 KiB block per 4
@@ -881,7 +895,7 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
                 g.n_tiles = (uint32_t)P->h_gcm_tiles.size() - g.first_tile;
                 P->h_gcm_segs.push_back(g);
             }
-            if (pass == 1) P->n_gcm_tiles_aes = (uint32_t)P->h_gcm_tiles.size();
+            if (pass == 1) P->gcm.n_tiles_aes = (uint32_t)P->h_gcm_tiles.size();
         }
     }
     // decode lists
@@ -906,49 +920,28 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
     P->need_sizing = !all_caps;
     std::stable_sort(P->h_deflate.begin(), P->h_deflate.end(), [&](uint32_t a, uint32_t b) { return P->h_entries[a].comp_len > P->h_entries[b].comp_len; });
     std::stable_sort(P->h_xz.begin(), P->h_xz.end(), [&](uint32_t a, uint32_t b) { return P->h_entries[a].comp_len > P->h_entries[b].comp_len; });
-    // device arrays + upload
+    // device arrays + upload; entries, segments and keys get room even when there are none: kernels take their pointers
     CK(P->d_buf.reserve(P->buf_bytes));
     CK(P->d_entries.reserve(n)); CK(P->d_entries_init.reserve(n));
     CK(P->d_segs.reserve(P->h_segs.size()));
     CK(P->d_keys.reserve(P->h_keys.size()));
     int rc = st.upload(ctx, P->d_buf.p);
     if (rc) return rc;
-    if (!P->h_segs.empty()) CK(cudaMemcpyAsync(P->d_segs.p, P->h_segs.data(), P->h_segs.size() * sizeof(Segment), cudaMemcpyHostToDevice, ctx->stream));
-    if (!P->h_keys.empty()) CK(cudaMemcpyAsync(P->d_keys.p, P->h_keys.data(), P->h_keys.size() * sizeof(DevKeys), cudaMemcpyHostToDevice, ctx->stream));
-    if (!P->h_ctr_tiles.empty()) {
-        CK(P->d_ctr_tiles.reserve(P->h_ctr_tiles.size()));
-        CK(cudaMemcpyAsync(P->d_ctr_tiles.p, P->h_ctr_tiles.data(), P->h_ctr_tiles.size() * sizeof(CtrTile), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    for (int v = 0; v < 5; v++) {
-        if (P->h_tiles[v].empty()) continue;
-        CK(P->d_tiles[v].reserve(P->h_tiles[v].size()));
-        CK(cudaMemcpyAsync(P->d_tiles[v].p, P->h_tiles[v].data(), P->h_tiles[v].size() * sizeof(CipherTile), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    if (!P->h_deflate.empty()) {
-        CK(P->d_deflate.reserve(P->h_deflate.size()));
-        CK(cudaMemcpyAsync(P->d_deflate.p, P->h_deflate.data(), P->h_deflate.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    if (!P->h_xz.empty()) {
-        CK(P->d_xz.reserve(P->h_xz.size()));
-        CK(cudaMemcpyAsync(P->d_xz.p, P->h_xz.data(), P->h_xz.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    }
+    cudaStream_t s = ctx->stream;
+    CK(P->d_segs.upload(P->h_segs, s)); CK(P->d_keys.upload(P->h_keys, s));
+    CK(P->d_ctr_tiles.upload(P->h_ctr_tiles, s));
+    for (int v = 0; v < 4; v++) CK(P->d_tiles[v].upload(P->h_tiles[v], s));
+    CK(P->d_deflate.upload(P->h_deflate, s)); CK(P->d_xz.upload(P->h_xz, s));
     if (!P->h_gcm_segs.empty()) {
-        CK(P->d_gcm_segs.reserve(P->h_gcm_segs.size())); CK(P->d_gcm_tiles.reserve(P->h_gcm_tiles.size() + 1));
-        CK(P->d_gcm_refs.reserve(P->h_gcm_refs.size())); CK(P->d_gcm_pows.reserve(P->h_gcm_refs.size()));
-        CK(P->d_gcm_partial.reserve(P->h_gcm_tiles.size() + 1));
-        CK(cudaMemcpyAsync(P->d_gcm_segs.p, P->h_gcm_segs.data(), P->h_gcm_segs.size() * sizeof(gcm::GcmSeg), cudaMemcpyHostToDevice, ctx->stream));
-        if (!P->h_gcm_tiles.empty())
-            CK(cudaMemcpyAsync(P->d_gcm_tiles.p, P->h_gcm_tiles.data(), P->h_gcm_tiles.size() * sizeof(gcm::GcmTile), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(P->d_gcm_refs.p, P->h_gcm_refs.data(), P->h_gcm_refs.size() * sizeof(gcm::GcmKeyRef), cudaMemcpyHostToDevice, ctx->stream));
+        GcmDev& G = P->gcm;
+        G.n_segs = (uint32_t)P->h_gcm_segs.size(); G.n_tiles = (uint32_t)P->h_gcm_tiles.size(); G.n_keys = (uint32_t)P->h_gcm_refs.size();
+        CK(G.tiles.reserve(G.n_tiles + 1)); CK(G.partial.reserve(G.n_tiles + 1)); CK(G.pows.reserve(G.n_keys));
+        CK(G.segs.upload(P->h_gcm_segs, s)); CK(G.tiles.upload(P->h_gcm_tiles, s)); CK(G.refs.upload(P->h_gcm_refs, s));
     }
     if (P->n_crc) {
-        const size_t nt = P->h_crc_tiles.size();
-        CK(P->d_crc_tiles.reserve(nt)); CK(P->d_crc_first.reserve(P->n_crc)); CK(P->d_crc_expect.reserve(P->n_crc));
-        CK(P->d_crc_entry.reserve(P->n_crc)); CK(P->d_crc_raw.reserve(nt)); CK(P->d_crc_val.reserve(P->n_crc)); CK(P->d_crc_broken.reserve(1));
-        CK(cudaMemcpyAsync(P->d_crc_tiles.p, P->h_crc_tiles.data(), nt * sizeof(CrcTile), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(P->d_crc_first.p, P->h_crc_first.data(), P->n_crc * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(P->d_crc_expect.p, P->h_crc_expect.data(), P->n_crc * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(P->d_crc_entry.p, P->h_crc_entry.data(), P->n_crc * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_crc_tiles.upload(P->h_crc_tiles, s)); CK(P->d_crc_first.upload(P->h_crc_first, s));
+        CK(P->d_crc_expect.upload(P->h_crc_expect, s)); CK(P->d_crc_entry.upload(P->h_crc_entry, s));
+        CK(P->d_crc_raw.reserve(P->h_crc_tiles.size())); CK(P->d_crc_val.reserve(P->n_crc)); CK(P->d_crc_broken.reserve(1));
     }
     CK(ctx->sync());   // the borrowed host spans may go away after this call
     return PNA_OK;
@@ -988,9 +981,8 @@ static int decode_layout_out(pna_plan* P) {
         }
         P->h_xz_win_begin.push_back((uint32_t)P->h_xz_map.size());
         if (!P->h_xz_map.empty()) {
-            CK(P->d_xz_map.reserve(P->h_xz_map.size())); CK(P->d_xz_wins.reserve(P->h_xz_map.size())); CK(P->d_xz_win_begin.reserve(P->h_xz_win_begin.size()));
-            CK(cudaMemcpyAsync(P->d_xz_map.p, P->h_xz_map.data(), P->h_xz_map.size() * sizeof(uint2), cudaMemcpyHostToDevice, ctx->stream));
-            CK(cudaMemcpyAsync(P->d_xz_win_begin.p, P->h_xz_win_begin.data(), P->h_xz_win_begin.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+            CK(P->d_xz_map.upload(P->h_xz_map, ctx->stream)); CK(P->d_xz_win_begin.upload(P->h_xz_win_begin, ctx->stream));
+            CK(P->d_xz_wins.reserve(P->h_xz_map.size()));
         }
     }
     // deflate: streams of the two-stage path with their literal / record arenas (sizes from the now final capacities)
@@ -1007,18 +999,13 @@ static int decode_layout_out(pna_plan* P) {
         }
         const size_t ni = P->h_inf.size();
         if (ni) {
-            CK(P->d_inf.reserve(ni)); CK(P->d_inf_lits.reserve(lit + 256)); CK(P->d_inf_recs.reserve(rec + 32));
+            CK(P->d_inf.upload(P->h_inf, ctx->stream)); CK(P->d_inf_lits.reserve(lit + 256)); CK(P->d_inf_recs.reserve(rec + 32));
             CK(P->d_inf_blocks.reserve(ni)); CK(P->d_inf_ze.reserve(ni)); CK(P->d_inf_tr.reserve(ni));
-            CK(cudaMemcpyAsync(P->d_inf.p, P->h_inf.data(), ni * sizeof(inf::InfStream), cudaMemcpyHostToDevice, ctx->stream));
         }
-        if (!P->h_deflate_big.empty())
-            CK(cudaMemcpyAsync(P->d_deflate.p, P->h_deflate_big.data(), P->h_deflate_big.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_deflate.upload(P->h_deflate_big, ctx->stream));   // a subset of h_deflate: fits
     }
-    if (!P->h_copy.empty()) {
-        CK(P->d_copy.reserve(P->h_copy.size()));
-        CK(cudaMemcpyAsync(P->d_copy.p, P->h_copy.data(), P->h_copy.size() * sizeof(CopyJob), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    CK(cudaMemcpyAsync(P->d_entries_init.p, P->h_entries.data(), P->n * sizeof(EntryRec), cudaMemcpyHostToDevice, ctx->stream));
+    CK(P->d_copy.upload(P->h_copy, ctx->stream));
+    CK(P->d_entries_init.upload(P->h_entries, ctx->stream));
     return PNA_OK;
 }
 
@@ -1032,64 +1019,61 @@ __global__ void crc_check_kernel(const uint32_t* __restrict__ crc, const uint32_
 static int launch_crc(pna_plan* P) {
     pna_ctx* ctx = P->ctx;
     if (!P->n_crc) return PNA_OK;
-    const uint32_t nt = (uint32_t)P->h_crc_tiles.size();
     CK(cudaMemsetAsync(P->d_crc_broken.p, 0, sizeof(uint32_t), ctx->stream));
-    launch_crc_tiles(ctx->stream, ctx->sm_count, P->d_buf.p, P->d_crc_tiles.p, nt, ctx->d_crc, P->d_crc_raw.p);
-    LAUNCHED();
-    crc_combine_kernel<<<(P->n_crc + 127) / 128, 128, 0, ctx->stream>>>(P->d_crc_tiles.p, P->d_crc_raw.p, P->d_crc_first.p, P->n_crc, nt,
-                                                                       ctx->d_crc, P->d_crc_val.p);
-    LAUNCHED();
+    const int rc = launch_chunk_crc(ctx, P->d_buf.p, P->d_crc_tiles.p, (uint32_t)P->h_crc_tiles.size(), P->d_crc_raw.p, P->d_crc_first.p,
+                                    P->n_crc, P->d_crc_val.p);
+    if (rc) return rc;
     crc_check_kernel<<<(P->n_crc + 127) / 128, 128, 0, ctx->stream>>>(P->d_crc_val.p, P->d_crc_expect.p, P->d_crc_entry.p, P->d_entries.p,
                                                                      P->n_crc, P->d_crc_broken.p);
     LAUNCHED();
     return PNA_OK;
 }
 
+// GCM STREAM in either direction over the segments of G, read from `src` through `segs` and written to `dst`: H and its
+// powers per key, CTR and partial GHASH over the AES tiles and then the Camellia tiles, and the tags, which decryption checks
+// (a mismatch fails the entry in `entries`) and encryption writes behind each segment in `dst`
+template <bool DECRYPT>
+static int launch_gcm(pna_ctx* ctx, const GcmDev& G, const uint8_t* src, const Segment* segs, uint8_t* dst, EntryRec* entries,
+                      const DevKeys* keys) {
+    if (!G.n_segs) return PNA_OK;
+    const uint32_t nk = G.n_keys, ns = G.n_segs, nt = G.n_tiles, na = G.n_tiles_aes;
+    gcm::gcm_setup_kernel<<<(nk + 127) / 128, 128, 0, ctx->stream>>>(G.refs.p, nk, keys, ctx->d_aes, ctx->d_cam, G.pows.p);
+    LAUNCHED();
+    const uint32_t cap = (uint32_t)ctx->sm_count * 3;
+    if (na) {
+        gcm::gcm_tiles_kernel<1, DECRYPT><<<std::min<uint32_t>((na + gcm::gcm_tile_warps<1>() - 1) / gcm::gcm_tile_warps<1>(), (uint32_t)ctx->sm_count), gcm::gcm_tile_warps<1>() * 32,
+                                            gcm::gcm_tiles_smem<1>(), ctx->stream>>>(src, segs, dst, G.segs.p, G.tiles.p, na, keys, G.pows.p, ctx->d_aes, ctx->d_cam,
+                                                                                     G.partial.p);
+        LAUNCHED();
+    }
+    if (nt > na) {
+        gcm::gcm_tiles_kernel<2, DECRYPT><<<std::min<uint32_t>((nt - na + gcm::gcm_tile_warps<2>() - 1) / gcm::gcm_tile_warps<2>(), cap), gcm::gcm_tile_warps<2>() * 32,
+                                            gcm::gcm_tiles_smem<2>(), ctx->stream>>>(src, segs, dst, G.segs.p, G.tiles.p + na, nt - na, keys, G.pows.p, ctx->d_aes,
+                                                                                     ctx->d_cam, G.partial.p + na);
+        LAUNCHED();
+    }
+    gcm::gcm_finish_kernel<DECRYPT><<<(ns + 127) / 128, 128, 0, ctx->stream>>>(src, segs, entries, G.segs.p, ns, keys, G.pows.p, ctx->d_aes, ctx->d_cam,
+                                                                               G.partial.p, DECRYPT ? nullptr : dst);
+    LAUNCHED();
+    return PNA_OK;
+}
+
 static int launch_cipher(pna_plan* P) {
     pna_ctx* ctx = P->ctx;
-    const int aes_smem = 256 * 32 * 4 + 256, cam_smem = 2 * 2048 * 4;
     if (const uint32_t nt = (uint32_t)P->h_ctr_tiles.size()) {
         aes_ctr_tiles_kernel<<<std::min<uint32_t>(nt, (uint32_t)ctx->sm_count), AES_CTR_THREADS, AES_CTR_TILES_SMEM, ctx->stream>>>(
             P->d_buf.p, P->d_segs.p, P->d_entries.p, P->d_ctr_tiles.p, nt, P->d_keys.p, ctx->d_aes);
         LAUNCHED();
     }
-    for (int v = 0; v < 5; v++) {
+    for (int v = 0; v < 4; v++) {
         const uint32_t nt = (uint32_t)P->h_tiles[v].size();
         if (!nt) continue;
-        const uint32_t grid = std::min<uint32_t>(nt, (uint32_t)ctx->sm_count * (v == 2 ? 4 : 6));
-#define ARGS P->d_buf.p, P->d_segs.p, P->d_entries.p, P->d_tiles[v].p, nt, P->d_keys.p, ctx->d_aes, ctx->d_cam
-        switch (v) {
-            case 0: decrypt_tiles_kernel<0, 1><<<grid, 256, 0, ctx->stream>>>(ARGS); break;
-            case 2: decrypt_tiles_kernel<1, 0><<<grid, 256, aes_smem, ctx->stream>>>(ARGS); break;
-            case 3: decrypt_tiles_kernel<2, 1><<<grid, 256, cam_smem, ctx->stream>>>(ARGS); break;
-            case 4: decrypt_tiles_kernel<2, 0><<<grid, 256, cam_smem, ctx->stream>>>(ARGS); break;
-        }
-#undef ARGS
+        const auto decrypt_tiles = DECRYPT_TILES[v].fn;
+        decrypt_tiles<<<std::min<uint32_t>(nt, (uint32_t)ctx->sm_count * (v == 1 ? 4 : 6)), 256, DECRYPT_TILES[v].smem, ctx->stream>>>(
+            P->d_buf.p, P->d_segs.p, P->d_entries.p, P->d_tiles[v].p, nt, P->d_keys.p, ctx->d_aes, ctx->d_cam);
         LAUNCHED();
     }
-    if (!P->h_gcm_segs.empty()) {
-        const uint32_t nk = (uint32_t)P->h_gcm_refs.size(), ns = (uint32_t)P->h_gcm_segs.size();
-        const uint32_t nt = (uint32_t)P->h_gcm_tiles.size(), na = P->n_gcm_tiles_aes;
-        gcm::gcm_setup_kernel<<<(nk + 127) / 128, 128, 0, ctx->stream>>>(P->d_gcm_refs.p, nk, P->d_keys.p, ctx->d_aes, ctx->d_cam, P->d_gcm_pows.p);
-        LAUNCHED();
-        const uint32_t cap = (uint32_t)ctx->sm_count * 3;
-        if (na) {
-            gcm::gcm_tiles_kernel<1, true><<<std::min<uint32_t>((na + gcm::gcm_tile_warps<1>() - 1) / gcm::gcm_tile_warps<1>(), (uint32_t)ctx->sm_count), gcm::gcm_tile_warps<1>() * 32,
-                                             gcm::gcm_tiles_smem<1>(), ctx->stream>>>(P->d_buf.p, P->d_segs.p, P->d_buf.p, P->d_gcm_segs.p,
-                P->d_gcm_tiles.p, na, P->d_keys.p, P->d_gcm_pows.p, ctx->d_aes, ctx->d_cam, P->d_gcm_partial.p);
-            LAUNCHED();
-        }
-        if (nt > na) {
-            gcm::gcm_tiles_kernel<2, true><<<std::min<uint32_t>((nt - na + gcm::gcm_tile_warps<2>() - 1) / gcm::gcm_tile_warps<2>(), cap), gcm::gcm_tile_warps<2>() * 32,
-                                             gcm::gcm_tiles_smem<2>(), ctx->stream>>>(P->d_buf.p, P->d_segs.p, P->d_buf.p, P->d_gcm_segs.p,
-                P->d_gcm_tiles.p + na, nt - na, P->d_keys.p, P->d_gcm_pows.p, ctx->d_aes, ctx->d_cam, P->d_gcm_partial.p + na);
-            LAUNCHED();
-        }
-        gcm::gcm_finish_kernel<true><<<(ns + 127) / 128, 128, 0, ctx->stream>>>(P->d_buf.p, P->d_segs.p, P->d_entries.p, P->d_gcm_segs.p, ns, P->d_keys.p,
-                                                                                P->d_gcm_pows.p, ctx->d_aes, ctx->d_cam, P->d_gcm_partial.p, nullptr);
-        LAUNCHED();
-    }
-    return PNA_OK;
+    return launch_gcm<true>(ctx, P->gcm, P->d_buf.p, P->d_segs.p, P->d_buf.p, P->d_entries.p, P->d_keys.p);
 }
 
 static int launch_zstd_front(pna_plan* P, bool with_count) {   // scan .. resolve
@@ -1213,8 +1197,7 @@ static int launch_inflate(pna_plan* P, int size_only) {
         if (!nd) return PNA_OK;
         std::vector<inf::InfStream> all(nd);
         for (uint32_t k = 0; k < nd; k++) all[k] = {P->h_deflate[k], 0u, 0ull, 0ull};
-        CK(P->d_inf.reserve(nd));
-        CK(cudaMemcpyAsync(P->d_inf.p, all.data(), nd * sizeof(inf::InfStream), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_inf.upload(all, ctx->stream));
         inf::inflate_tokens_kernel<<<(nd + inf::TOKEN_CTA - 1) / inf::TOKEN_CTA, inf::TOKEN_CTA, inf::TOKEN_SMEM_BYTES, ctx->stream>>>(
             P->d_buf.p, P->d_entries.p, P->d_inf.p, nd, nullptr, nullptr, nullptr, nullptr, nullptr, 1);
         LAUNCHED();
@@ -1259,12 +1242,11 @@ static int decode_prepare(pna_plan* P) {
     pna_ctx* ctx = P->ctx;
     int rc;
     const uint32_t nz = (uint32_t)P->h_ze.size();
-    CK(cudaMemcpyAsync(P->d_entries.p, P->h_entries.data(), P->n * sizeof(EntryRec), cudaMemcpyHostToDevice, ctx->stream));
+    CK(P->d_entries.upload(P->h_entries, ctx->stream));
     if ((rc = launch_crc(P))) return rc;
     if ((rc = launch_cipher(P))) return rc;
     if (nz) {
-        CK(P->d_ze.reserve(nz));
-        CK(cudaMemcpyAsync(P->d_ze.p, P->h_ze.data(), nz * sizeof(zs::ZEntry), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_ze.upload(P->h_ze, ctx->stream));
         // LZ stage order: longest compressed streams first (one CTA per entry, dispatched in grid order)
         std::vector<uint32_t> lz_order(nz);
         for (uint32_t i = 0; i < nz; i++) lz_order[i] = i;
@@ -1279,7 +1261,7 @@ static int decode_prepare(pna_plan* P) {
         P->n_blocks = (uint32_t)nb;
         CK(P->d_blocks.reserve(nb)); CK(P->d_walk.reserve(nb));
         CK(P->d_seq_order.reserve(nb)); CK(P->d_lit_order.reserve(nb)); CK(P->d_counts.reserve(8));
-        CK(cudaMemcpyAsync(P->d_ze.p, P->h_ze.data(), nz * sizeof(zs::ZEntry), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_ze.upload(P->h_ze, ctx->stream));
         if ((rc = launch_zstd_front(P, false))) return rc;
         CK(cudaMemcpyAsync(P->h_ze.data(), P->d_ze.p, nz * sizeof(zs::ZEntry), cudaMemcpyDeviceToHost, ctx->stream));
         CK(ctx->sync());
@@ -1322,8 +1304,7 @@ static int decode_prepare(pna_plan* P) {
             }
         }
         if (!P->h_pj_segs.empty()) {
-            CK(P->d_pj_segs.reserve(P->h_pj_segs.size()));
-            CK(cudaMemcpyAsync(P->d_pj_segs.p, P->h_pj_segs.data(), P->h_pj_segs.size() * sizeof(zs::PjSeg), cudaMemcpyHostToDevice, ctx->stream));
+            CK(P->d_pj_segs.upload(P->h_pj_segs, ctx->stream));
             CK(P->d_pj_ptr.reserve((size_t)P->pj_max_blocks * zs::BLOCK_MAX + 64));
             CK(P->d_pj_cpos.reserve((size_t)P->pj_max_blocks * zs::PJ_MAX_CHUNKS));
             CK(P->d_pj_flags.reserve(P->h_pj_segs.size() * zs::PJ_MAX_ROUNDS));
@@ -1337,15 +1318,13 @@ static int decode_prepare(pna_plan* P) {
             for (uint32_t f = 0; f < P->h_ze[zi].n_frames; f++) unit_order.push_back(P->h_ze[zi].unit_begin + f);
         }
         CK(P->d_lz_order.reserve(nu + 1)); CK(P->d_lz_units.reserve(nu + 1));
-        if (!unit_order.empty()) CK(cudaMemcpyAsync(P->d_lz_order.p, unit_order.data(), unit_order.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_lz_order.upload(unit_order, ctx->stream));
         const uint32_t n_regular_units = (uint32_t)unit_order.size();
         P->lit_total = lit; P->seq_total = seq;
         CK(P->d_lits.reserve(lit + 256));
         CK(P->d_seqs.reserve(seq + 32));
-        CK(P->d_lit_base.reserve(P->n)); CK(P->d_seq_base.reserve(P->n));
-        CK(cudaMemcpyAsync(P->d_lit_base.p, lb.data(), P->n * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(P->d_seq_base.p, sb.data(), P->n * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(P->d_ze.p, P->h_ze.data(), nz * sizeof(zs::ZEntry), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_lit_base.upload(lb, ctx->stream)); CK(P->d_seq_base.upload(sb, ctx->stream));
+        CK(P->d_ze.upload(P->h_ze, ctx->stream));
         zs::zstd_units_kernel<<<(nz + 127) / 128, 128, 0, ctx->stream>>>(P->d_ze.p, nz, P->d_blocks.p, P->d_lz_units.p);
         LAUNCHED();
         CK(ctx->sync());   // lb/sb/unit_order are locals
@@ -1383,6 +1362,17 @@ __global__ void set_layout_kernel(EntryRec* entries, const uint64_t* __restrict_
 }
 
 #define STAGE(i) do { if (P->ev_ready) CK(cudaEventRecord(P->ev[i], ctx->stream)); } while (0)
+// the plan's stage-timing events, on its first run: from the context's pool (~pna_plan gives them back) or new
+static int lease_stage_events(pna_plan* P) {
+    pna_ctx* ctx = P->ctx;
+    if (P->ev_ready) return PNA_OK;
+    for (auto& e : P->ev) {
+        if (!ctx->ev_pool.empty()) { e = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); }
+        else CK(cudaEventCreate(&e));
+    }
+    P->ev_ready = true;
+    return PNA_OK;
+}
 // fresh = true: full pipeline from the pristine entry table (every run after the first).
 // fresh = false: continue right after decode_prepare(), which already decrypted and scanned (and, when it had
 // to size outputs, entropy-decoded) on the live table -- so a one-shot pna_cuda_decode_batch does no work twice.
@@ -1390,13 +1380,7 @@ static int decode_launch_all(pna_plan* P, bool fresh) {
     pna_ctx* ctx = P->ctx;
     int rc;
     const uint64_t l0 = ctx->launches;
-    if (!P->ev_ready) {
-        for (auto& e : P->ev) {
-            if (!ctx->ev_pool.empty()) { e = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); }
-            else CK(cudaEventCreate(&e));
-        }
-        P->ev_ready = true;
-    }
+    if ((rc = lease_stage_events(P))) return rc;
     if (fresh) {
         CK(cudaMemcpyAsync(P->d_entries.p, P->d_entries_init.p, P->n * sizeof(EntryRec), cudaMemcpyDeviceToDevice, ctx->stream));
         STAGE(0);
@@ -1414,8 +1398,7 @@ static int decode_launch_all(pna_plan* P, bool fresh) {
     } else {
         std::vector<uint64_t> oc(2 * (size_t)P->n);
         for (uint32_t i = 0; i < P->n; i++) { oc[2 * i] = P->h_entries[i].out_off; oc[2 * i + 1] = P->h_entries[i].out_cap; }
-        CK(P->d_layout.reserve(oc.size()));
-        CK(cudaMemcpyAsync(P->d_layout.p, oc.data(), oc.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+        CK(P->d_layout.upload(oc, ctx->stream));
         set_layout_kernel<<<(P->n + 127) / 128, 128, 0, ctx->stream>>>(P->d_entries.p, P->d_layout.p, P->n);
         LAUNCHED();
         CK(ctx->sync());   // oc is a local
@@ -1762,25 +1745,15 @@ extern "C" int pna_cuda_ecb(pna_ctx* ctx, int encryption, int encrypt, const uin
         memcpy(dk.cam_ek, ck.ek, sizeof ck.ek); memcpy(dk.cam_dk, ck.dk, sizeof ck.dk);
     }
     DevArr<uint8_t> d_in, d_out; DevArr<DevKeys> d_key;
-    CK(d_in.reserve(nb * 16 + 64)); CK(d_out.reserve(nb * 16)); CK(d_key.reserve(1));
-    int rc = PNA_OK;
-    cudaError_t e;
-    if ((e = cudaMemcpyAsync(d_in.p, in, nb * 16, cudaMemcpyHostToDevice, ctx->stream)) != cudaSuccess ||
-        (e = cudaMemcpyAsync(d_key.p, &dk, sizeof dk, cudaMemcpyHostToDevice, ctx->stream)) != cudaSuccess) {
-        ctx->fail("ecb upload", e); rc = PNA_E_CUDA;
-    }
-    if (rc == PNA_OK) {
-        const uint32_t grid = (uint32_t)std::min<uint64_t>((nb + 255) / 256, (uint64_t)ctx->sm_count * 4);
-        ecb_kernel<<<grid, 256, 256 * 32 * 4 + 256, ctx->stream>>>(encryption, encrypt, d_key.p, ctx->d_aes, ctx->d_cam, d_in.p, nb, d_out.p);
-        ctx->launches++;
-        if ((e = cudaGetLastError()) != cudaSuccess ||
-            (e = cudaMemcpyAsync(out, d_out.p, nb * 16, cudaMemcpyDeviceToHost, ctx->stream)) != cudaSuccess ||
-            (e = ctx->sync()) != cudaSuccess) {
-            ctx->fail("ecb run", e); rc = PNA_E_CUDA;
-        }
-    }
-    d_in.release(); d_out.release(); d_key.release();
-    return rc;
+    CK(d_in.reserve(nb * 16 + 64)); CK(d_out.reserve(nb * 16));
+    CK(cudaMemcpyAsync(d_in.p, in, nb * 16, cudaMemcpyHostToDevice, ctx->stream));
+    CK(d_key.upload(&dk, 1, ctx->stream));
+    const uint32_t grid = (uint32_t)std::min<uint64_t>((nb + 255) / 256, (uint64_t)ctx->sm_count * 4);
+    ecb_kernel<<<grid, 256, ECB_SMEM, ctx->stream>>>(encryption, encrypt, d_key.p, ctx->d_aes, ctx->d_cam, d_in.p, nb, d_out.p);
+    LAUNCHED();
+    CK(cudaMemcpyAsync(out, d_out.p, nb * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx->sync());
+    return PNA_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -32,23 +32,20 @@ struct EncodePlan {
     // GCM STREAM: segment / tile slots from the compressed-length bounds (AES slots first, then Camellia)
     std::vector<GcmSlot> h_gcm_slots;
     std::vector<gcm::GcmKeyRef> h_gcm_refs;
-    uint32_t n_gcm_tiles = 0, n_gcm_tiles_aes = 0;
     DevArr<GcmSlot> d_gcm_slots;
-    DevArr<gcm::GcmKeyRef> d_gcm_refs;
-    DevArr<gcm::GcmSeg> d_gcm_segs;
-    DevArr<gcm::GcmTile> d_gcm_tiles;
-    DevArr<gcm::GcmPow> d_gcm_pows;
-    DevArr<gcm::G128> d_gcm_partial;
+    GcmDev gcm;
 };
 void destroy(EncodePlan* p) { delete p; }
+// cipher kernels by slot: h_tiles / d_tiles (AES-CTR with AES_CTR_THREADS, one CTA per SM) and h_cbc / d_cbc
+static const CipherKernel<decltype(&encrypt_tiles_kernel<0>)> ENCRYPT_TILES[3] = {
+    {encrypt_tiles_kernel<0>, 0}, {encrypt_tiles_kernel<1>, AES_CTR_SMEM}, {encrypt_tiles_kernel<2>, CAM_SMEM}};
+static const CipherKernel<decltype(&cbc_encrypt_kernel<1>)> CBC_ENCRYPT[2] = {{cbc_encrypt_kernel<1>, AES_SMEM}, {cbc_encrypt_kernel<2>, CAM_SMEM}};
 bool init_attributes() {
-    const int aes_smem = 256 * 32 * 4, cam_smem = 2 * 2048 * 4;
-    return cudaFuncSetAttribute(lz_match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MATCH_SMEM_BYTES) == cudaSuccess &&
-           cudaFuncSetAttribute(xz_encode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)xz_enc_smem_bytes(xz::ENC_LC_MAX)) == cudaSuccess &&
-           cudaFuncSetAttribute(encrypt_tiles_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, AES_CTR_SMEM) == cudaSuccess &&
-           cudaFuncSetAttribute(encrypt_tiles_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, cam_smem) == cudaSuccess &&
-           cudaFuncSetAttribute(cbc_encrypt_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, aes_smem) == cudaSuccess &&
-           cudaFuncSetAttribute(cbc_encrypt_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, cam_smem) == cudaSuccess;
+    bool ok = cudaFuncSetAttribute(lz_match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MATCH_SMEM_BYTES) == cudaSuccess &&
+              cudaFuncSetAttribute(xz_encode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)xz_enc_smem_bytes(xz::ENC_LC_MAX)) == cudaSuccess;
+    for (const auto& k : ENCRYPT_TILES) ok = ok && k.opt_in();
+    for (const auto& k : CBC_ENCRYPT) ok = ok && k.opt_in();
+    return ok;
 }
 }}  // namespace pna::enc
 
@@ -214,26 +211,26 @@ static int encode_plan_build(pna_ctx* ctx, const pna_encode_desc* descs, uint32_
             const uint64_t cb = enc_comp_bound(e.compression, e.plain_len), S = e.gcm_seg_size;
             const uint64_t max_segs = cb / S + 1;
             const uint64_t tps = ((S + 15) / 16 + gcm::GCM_TILE_BLOCKS - 1) / gcm::GCM_TILE_BLOCKS;
-            if (E->h_gcm_slots.size() + max_segs > 0x7FFFFFF0ull || (uint64_t)E->n_gcm_tiles + max_segs * tps > 0x7FFFFFF0ull) return PNA_E_OOM;
+            if (E->h_gcm_slots.size() + max_segs > 0x7FFFFFF0ull || (uint64_t)E->gcm.n_tiles + max_segs * tps > 0x7FFFFFF0ull) return PNA_E_OOM;
             e.gcm_slot_begin = (uint32_t)E->h_gcm_slots.size();
-            e.gcm_tile_begin = E->n_gcm_tiles;
+            e.gcm_tile_begin = E->gcm.n_tiles;
             e.gcm_tiles_per_seg = (uint32_t)tps;
             e.gcm_pow_idx = (uint32_t)E->h_gcm_refs.size();
             E->h_gcm_refs.push_back({e.key_idx, (uint32_t)e.encryption});
             for (uint64_t j = 0; j < max_segs; j++) E->h_gcm_slots.push_back({i, (uint32_t)j});
-            E->n_gcm_tiles += (uint32_t)(max_segs * tps);
+            E->gcm.n_tiles += (uint32_t)(max_segs * tps);
         }
-        if (pass == 1) E->n_gcm_tiles_aes = E->n_gcm_tiles;
+        if (pass == 1) E->gcm.n_tiles_aes = E->gcm.n_tiles;
     }
     E->n_pieces = piece_cur;
     E->out_bytes = out_cur;
     E->seq_total = nsegs_total * enc::SEG_SEQ_MAX;
     if (crc_bodies > 0xFFFFFFF0ull || E->h_crc_src.size() > 0xFFFFFFF0ull) return PNA_E_OOM;
-    // device arrays + upload
+    // device arrays + upload; segments and keys get room even when there are none: kernels take their pointers
     CK(E->d_work.reserve(E->work_bytes)); CK(E->d_out.reserve(E->out_bytes + 256));
     CK(E->d_entries.reserve(n)); CK(E->d_entries_init.reserve(n));
     CK(E->d_segs.reserve(nsegs_total)); CK(E->d_seqs.reserve(E->seq_total + 8)); CK(E->d_pieces.reserve(piece_cur + 1));
-    CK(E->d_keys.reserve(E->h_keys.size())); CK(E->d_tables.reserve(1));
+    CK(E->d_keys.reserve(E->h_keys.size()));
     {
         // Upload of the plaintext.  A cudaMemcpyAsync costs the host 5-10 us whatever its size, which is what a group of
         // thousands of small files is made of -- so runs of entries whose host spans are exactly adjacent (files packed into one
@@ -270,8 +267,7 @@ static int encode_plan_build(pna_ctx* ctx, const pna_encode_desc* descs, uint32_
                     at += descs[k].plain.len;
                 }
             }
-            CK(E->d_stage_jobs.reserve(jobs.size()));
-            CK(cudaMemcpyAsync(E->d_stage_jobs.p, jobs.data(), jobs.size() * sizeof(CopyJob), cudaMemcpyHostToDevice, ctx->stream));
+            CK(E->d_stage_jobs.upload(jobs, ctx->stream));
             const uint32_t grid = std::min<uint32_t>(((uint32_t)jobs.size() + 7) / 8, (uint32_t)ctx->sm_count * 8);
             copy_jobs_kernel<<<grid, 256, 0, ctx->stream>>>(E->d_work.p, E->d_stage.p, E->d_stage_jobs.p, (uint32_t)jobs.size());
             LAUNCHED();
@@ -279,36 +275,23 @@ static int encode_plan_build(pna_ctx* ctx, const pna_encode_desc* descs, uint32_
             E->d_stage.release();
         }
     }
-    CK(cudaMemcpyAsync(E->d_entries_init.p, E->h_entries.data(), n * sizeof(EncEntry), cudaMemcpyHostToDevice, ctx->stream));
-    if (nsegs_total) CK(cudaMemcpyAsync(E->d_segs.p, E->h_segs.data(), nsegs_total * sizeof(enc::SegRec), cudaMemcpyHostToDevice, ctx->stream));
-    if (!E->h_keys.empty()) CK(cudaMemcpyAsync(E->d_keys.p, E->h_keys.data(), E->h_keys.size() * sizeof(DevKeys), cudaMemcpyHostToDevice, ctx->stream));
+    cudaStream_t s = ctx->stream;
+    CK(E->d_entries_init.upload(E->h_entries, s)); CK(E->d_segs.upload(E->h_segs, s)); CK(E->d_keys.upload(E->h_keys, s));
     static enc::EncTables h_tables;
     static std::once_flag h_tables_once;   // plans are built concurrently by the host layer's worker threads
     std::call_once(h_tables_once, []() { enc::make_enc_tables(&h_tables); });
-    CK(cudaMemcpyAsync(E->d_tables.p, &h_tables, sizeof h_tables, cudaMemcpyHostToDevice, ctx->stream));
-    for (int v = 0; v < 3; v++) {
-        if (E->h_tiles[v].empty()) continue;
-        CK(E->d_tiles[v].reserve(E->h_tiles[v].size()));
-        CK(cudaMemcpyAsync(E->d_tiles[v].p, E->h_tiles[v].data(), E->h_tiles[v].size() * sizeof(CipherTile), cudaMemcpyHostToDevice, ctx->stream));
-    }
-    for (int v = 0; v < 2; v++) {
-        if (E->h_cbc[v].empty()) continue;
-        CK(E->d_cbc[v].reserve(E->h_cbc[v].size()));
-        CK(cudaMemcpyAsync(E->d_cbc[v].p, E->h_cbc[v].data(), E->h_cbc[v].size() * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-    }
+    CK(E->d_tables.upload(&h_tables, 1, s));
+    for (int v = 0; v < 3; v++) CK(E->d_tiles[v].upload(E->h_tiles[v], s));
+    for (int v = 0; v < 2; v++) CK(E->d_cbc[v].upload(E->h_cbc[v], s));
     if (!E->h_gcm_slots.empty()) {
-        const size_t ns = E->h_gcm_slots.size();
-        CK(E->d_gcm_slots.reserve(ns)); CK(E->d_gcm_segs.reserve(ns)); CK(E->d_gcm_refs.reserve(E->h_gcm_refs.size()));
-        CK(E->d_gcm_pows.reserve(E->h_gcm_refs.size())); CK(E->d_gcm_tiles.reserve(E->n_gcm_tiles + 1)); CK(E->d_gcm_partial.reserve(E->n_gcm_tiles + 1));
-        CK(cudaMemcpyAsync(E->d_gcm_slots.p, E->h_gcm_slots.data(), ns * sizeof(enc::GcmSlot), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(E->d_gcm_refs.p, E->h_gcm_refs.data(), E->h_gcm_refs.size() * sizeof(gcm::GcmKeyRef), cudaMemcpyHostToDevice, ctx->stream));
+        GcmDev& G = E->gcm;
+        G.n_segs = (uint32_t)E->h_gcm_slots.size(); G.n_keys = (uint32_t)E->h_gcm_refs.size();
+        CK(E->d_gcm_slots.upload(E->h_gcm_slots, s)); CK(G.refs.upload(E->h_gcm_refs, s));
+        CK(G.segs.reserve(G.n_segs)); CK(G.pows.reserve(G.n_keys)); CK(G.tiles.reserve(G.n_tiles + 1)); CK(G.partial.reserve(G.n_tiles + 1));
     }
-    const size_t nt = E->h_crc_src.size(), nb = E->h_crc_first.size();
-    if (nt) {
-        CK(E->d_crc_src.reserve(nt)); CK(E->d_crc_tiles.reserve(nt)); CK(E->d_crc_raw.reserve(nt));
-        CK(E->d_crc_first.reserve(nb)); CK(E->d_crc_val.reserve(nb));
-        CK(cudaMemcpyAsync(E->d_crc_src.p, E->h_crc_src.data(), nt * sizeof(enc::CrcTileSrc), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(E->d_crc_first.p, E->h_crc_first.data(), nb * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+    if (!E->h_crc_src.empty()) {
+        CK(E->d_crc_src.upload(E->h_crc_src, s)); CK(E->d_crc_first.upload(E->h_crc_first, s));
+        CK(E->d_crc_tiles.reserve(E->h_crc_src.size())); CK(E->d_crc_raw.reserve(E->h_crc_src.size())); CK(E->d_crc_val.reserve(E->h_crc_first.size()));
     }
     {   // register value after the chunk type: chunk CRC covers type || data (lib/src/format/chunk.rs:7-12)
         uint32_t c = 0xFFFFFFFFu;
@@ -326,13 +309,8 @@ static int encode_launch_all(pna_plan* P) {
     EncodePlan* E = P->enc;
     const uint64_t l0 = ctx->launches;
     const uint32_t n = P->n, nsegs = (uint32_t)E->h_segs.size();
-    if (!P->ev_ready) {
-        for (auto& e : P->ev) {
-            if (!ctx->ev_pool.empty()) { e = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); }
-            else CK(cudaEventCreate(&e));
-        }
-        P->ev_ready = true;
-    }
+    int rc = lease_stage_events(P);
+    if (rc) return rc;
     CK(cudaMemcpyAsync(E->d_entries.p, E->d_entries_init.p, n * sizeof(EncEntry), cudaMemcpyDeviceToDevice, ctx->stream));
     STAGE(0);
     if (nsegs) {
@@ -360,60 +338,35 @@ static int encode_launch_all(pna_plan* P) {
     enc::enc_layout_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(E->d_work.p, E->d_segs.p, E->d_entries.p, n, E->d_pieces.p);
     LAUNCHED();
     STAGE(3);
-    const int aes_smem = 256 * 32 * 4, cam_smem = 2 * 2048 * 4;
     for (int v = 0; v < 3; v++) {
         const uint32_t nt = (uint32_t)E->h_tiles[v].size();
         if (!nt) continue;
-        const uint32_t grid = std::min<uint32_t>(nt, (uint32_t)ctx->sm_count * (v == 1 ? 4 : 6));
-#define ARGS E->d_work.p, E->d_pieces.p, E->d_entries.p, E->d_tiles[v].p, nt, E->d_keys.p, ctx->d_aes, ctx->d_cam, E->d_out.p
-        if (v == 0) enc::encrypt_tiles_kernel<0><<<grid, 256, 0, ctx->stream>>>(ARGS);
-        else if (v == 1) enc::encrypt_tiles_kernel<1><<<std::min<uint32_t>(nt, (uint32_t)ctx->sm_count), AES_CTR_THREADS, AES_CTR_SMEM, ctx->stream>>>(ARGS);
-        else enc::encrypt_tiles_kernel<2><<<grid, 256, cam_smem, ctx->stream>>>(ARGS);
-#undef ARGS
+        const auto encrypt_tiles = enc::ENCRYPT_TILES[v].fn;
+        encrypt_tiles<<<std::min<uint32_t>(nt, (uint32_t)ctx->sm_count * (v == 1 ? 1 : 6)), v == 1 ? AES_CTR_THREADS : 256, enc::ENCRYPT_TILES[v].smem,
+                        ctx->stream>>>(E->d_work.p, E->d_pieces.p, E->d_entries.p, E->d_tiles[v].p, nt, E->d_keys.p, ctx->d_aes, ctx->d_cam, E->d_out.p);
         LAUNCHED();
     }
     for (int v = 0; v < 2; v++) {
         const uint32_t nc = (uint32_t)E->h_cbc[v].size();
         if (!nc) continue;
-#define ARGS E->d_work.p, E->d_pieces.p, E->d_entries.p, E->d_cbc[v].p, nc, E->d_keys.p, ctx->d_aes, ctx->d_cam, E->d_out.p
-        if (v == 0) enc::cbc_encrypt_kernel<1><<<(nc + 63) / 64, 64, aes_smem, ctx->stream>>>(ARGS);
-        else enc::cbc_encrypt_kernel<2><<<(nc + 63) / 64, 64, cam_smem, ctx->stream>>>(ARGS);
-#undef ARGS
+        const auto cbc_encrypt = enc::CBC_ENCRYPT[v].fn;
+        cbc_encrypt<<<(nc + 63) / 64, 64, enc::CBC_ENCRYPT[v].smem, ctx->stream>>>(E->d_work.p, E->d_pieces.p, E->d_entries.p, E->d_cbc[v].p, nc, E->d_keys.p,
+                                                                                 ctx->d_aes, ctx->d_cam, E->d_out.p);
         LAUNCHED();
     }
-    if (!E->h_gcm_slots.empty()) {
-        const uint32_t ns = (uint32_t)E->h_gcm_slots.size(), nk = (uint32_t)E->h_gcm_refs.size(), ntl = E->n_gcm_tiles, na = E->n_gcm_tiles_aes;
-        enc::gcm_enc_slots_kernel<<<(ns + 127) / 128, 128, 0, ctx->stream>>>(E->d_gcm_slots.p, ns, E->d_entries.p, E->d_gcm_segs.p, E->d_gcm_tiles.p, E->d_out.p);
+    if (const uint32_t ns = E->gcm.n_segs) {
+        enc::gcm_enc_slots_kernel<<<(ns + 127) / 128, 128, 0, ctx->stream>>>(E->d_gcm_slots.p, ns, E->d_entries.p, E->gcm.segs.p, E->gcm.tiles.p, E->d_out.p);
         LAUNCHED();
-        gcm::gcm_setup_kernel<<<(nk + 127) / 128, 128, 0, ctx->stream>>>(E->d_gcm_refs.p, nk, E->d_keys.p, ctx->d_aes, ctx->d_cam, E->d_gcm_pows.p);
-        LAUNCHED();
-        const uint32_t cap = (uint32_t)ctx->sm_count * 3;
-        if (na) {
-            gcm::gcm_tiles_kernel<1, false><<<std::min<uint32_t>((na + gcm::gcm_tile_warps<1>() - 1) / gcm::gcm_tile_warps<1>(), (uint32_t)ctx->sm_count), gcm::gcm_tile_warps<1>() * 32,
-                                              gcm::gcm_tiles_smem<1>(), ctx->stream>>>(E->d_work.p, E->d_pieces.p, E->d_out.p, E->d_gcm_segs.p,
-                E->d_gcm_tiles.p, na, E->d_keys.p, E->d_gcm_pows.p, ctx->d_aes, ctx->d_cam, E->d_gcm_partial.p);
-            LAUNCHED();
-        }
-        if (ntl > na) {
-            gcm::gcm_tiles_kernel<2, false><<<std::min<uint32_t>((ntl - na + gcm::gcm_tile_warps<2>() - 1) / gcm::gcm_tile_warps<2>(), cap), gcm::gcm_tile_warps<2>() * 32,
-                                              gcm::gcm_tiles_smem<2>(), ctx->stream>>>(E->d_work.p, E->d_pieces.p, E->d_out.p, E->d_gcm_segs.p,
-                E->d_gcm_tiles.p + na, ntl - na, E->d_keys.p, E->d_gcm_pows.p, ctx->d_aes, ctx->d_cam, E->d_gcm_partial.p + na);
-            LAUNCHED();
-        }
-        gcm::gcm_finish_kernel<false><<<(ns + 127) / 128, 128, 0, ctx->stream>>>(E->d_work.p, E->d_pieces.p, nullptr, E->d_gcm_segs.p, ns, E->d_keys.p,
-                                                                                 E->d_gcm_pows.p, ctx->d_aes, ctx->d_cam, E->d_gcm_partial.p, E->d_out.p);
-        LAUNCHED();
+        if ((rc = launch_gcm<false>(ctx, E->gcm, E->d_work.p, E->d_pieces.p, E->d_out.p, nullptr, E->d_keys.p))) return rc;
     }
     STAGE(4);
-    const uint32_t nt = (uint32_t)E->h_crc_src.size(), nb = (uint32_t)E->h_crc_first.size();
+    const uint32_t nt = (uint32_t)E->h_crc_src.size();
     if (nt) {
         enc::crc_clip_kernel<<<(nt + 127) / 128, 128, 0, ctx->stream>>>(E->d_crc_src.p, nt, E->d_entries.p, E->d_crc_tiles.p);
         LAUNCHED();
-        launch_crc_tiles(ctx->stream, ctx->sm_count, E->d_out.p, E->d_crc_tiles.p, nt, ctx->d_crc, E->d_crc_raw.p);
-        LAUNCHED();
-        crc_combine_kernel<<<(nb + 127) / 128, 128, 0, ctx->stream>>>(E->d_crc_tiles.p, E->d_crc_raw.p, E->d_crc_first.p, nb, nt, ctx->d_crc,
-                                                                     E->d_crc_val.p, E->fdat_init);
-        LAUNCHED();
+        if ((rc = launch_chunk_crc(ctx, E->d_out.p, E->d_crc_tiles.p, nt, E->d_crc_raw.p, E->d_crc_first.p, (uint32_t)E->h_crc_first.size(),
+                                   E->d_crc_val.p, E->fdat_init)))
+            return rc;
     }
     STAGE(5);
     for (int k = 6; k <= PNA_N_STAGES; k++) STAGE(k);
@@ -516,8 +469,7 @@ static int encode_plan_fetch_impl(pna_plan* P, pna_buf* out, uint32_t* fdat_crc_
                 for (uint64_t o = 0; o < e.out_len; o += PIECE)
                     jobs.push_back({(uint64_t)(out[i].ptr - lo) + o, e.out_off + o, std::min<uint64_t>(PIECE, e.out_len - o)});
             }
-            CK(E->d_stage.reserve(span + 256)); CK(E->d_stage_jobs.reserve(jobs.size()));
-            CK(cudaMemcpyAsync(E->d_stage_jobs.p, jobs.data(), jobs.size() * sizeof(CopyJob), cudaMemcpyHostToDevice, ctx->stream));
+            CK(E->d_stage.reserve(span + 256)); CK(E->d_stage_jobs.upload(jobs, ctx->stream));
             const uint32_t grid = std::min<uint32_t>(((uint32_t)jobs.size() + 7) / 8, (uint32_t)ctx->sm_count * 8);
             copy_jobs_kernel<<<grid, 256, 0, ctx->stream>>>(E->d_stage.p, E->d_out.p, E->d_stage_jobs.p, (uint32_t)jobs.size());
             LAUNCHED();

@@ -207,6 +207,9 @@ __global__ void __launch_bounds__(1024) zstd_order_kernel(const EntryRec* __rest
 // The kernel is not waiting on latency that a second chain could fill: with ONE warp per scheduler the integer pipe issues
 // a warp instruction every two cycles at best, the loop runs at 0.27 of a possible 0.5 IPC, and fewer active lanes per warp
 // means more warp instructions for the same sequences.  What would help is fewer instructions per sequence or smaller tables.
+// Fewer instructions (profiles/r3_seq_ab.log): the common path of the step loop is 112 static SASS instructions (73 ALU-pipe,
+// 22 IMAD, 10 memory, 7 control), against 184 before (110 / 45 / 11 / 17), and the stage went from 9.5 to 7.4 ms on the cfg2
+// shard (one B200, 1000 W limit, 1965 MHz).  The rare paths (second window, ring refill, escapes) are not counted.
 constexpr uint32_t SEQ_SLOTS = 22, SEQ_WARPS = 4;
 constexpr uint32_t SEQ_TAB_BYTES = TAB16_TOTAL * SEQ_SLOTS * SEQ_WARPS * sizeof(uint16_t);    // 225280
 constexpr uint32_t SEQ_SMEM_BYTES = SEQ_TAB_BYTES + SEQ_SLOTS * SEQ_WARPS * 64;               // + a 64-byte bitstream ring per block in flight
@@ -216,9 +219,10 @@ constexpr uint32_t SEQ_SMEM_BYTES = SEQ_TAB_BYTES + SEQ_SLOTS * SEQ_WARPS * 64; 
 // <= 3 words per window, so one conditional refill per window keeps groups (A>>2) and (A>>2)-1 resident and complete.
 struct RingBitSrc {
     uint32_t* ring;            // this lane's 16 words (64-byte aligned shared memory)
+    uint32_t rs;               // its shared-memory address: word k of the ring is at rs | (k & 15) * 4
     const uint32_t* words;     // arena start: nothing below it is fetched
     const uint32_t* gbase;     // 16-byte aligned group that holds the stream's first byte
-    uint32_t mis, b0;          // word phase of the stream start inside its group; bit offset inside its word
+    int32_t qoff;              // bit index from gbase of the bit below position 0: position p's top bit is p + qoff
     int32_t gl;                // lowest group loaded or in flight
     __device__ __forceinline__ void fetch(int32_t g) {
         const uint32_t* src = gbase + 4 * (int64_t)g;
@@ -229,23 +233,37 @@ struct RingBitSrc {
     }
     __device__ __forceinline__ void init(const uint32_t* w, uint64_t begin, int32_t pos) {
         words = w;
+#if defined(PNA_EMU)
+        rs = 0;
+#else
+        rs = (uint32_t)__cvta_generic_to_shared(ring);
+#endif
         const uint32_t* wb = w + (begin >> 2);
-        mis = (uint32_t)(reinterpret_cast<uintptr_t>(wb) >> 2) & 3u;
+        const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(wb) >> 2) & 3u;   // word phase of the start in its group
         gbase = wb - mis;
-        b0 = (uint32_t)(begin & 3) * 8;
-        const int32_t a = (((int32_t)b0 + pos - 1) >> 5) + (int32_t)mis;
-        gl = (a >> 2) - 3;
+        qoff = (int32_t)(mis * 32 + (uint32_t)(begin & 3) * 8) - 1;
+        gl = ((pos + qoff) >> 7) - 3;
         for (int32_t g = gl + 3; g >= gl; g--) fetch(g);
         cp_async_wait_all();
     }
     __device__ __forceinline__ uint64_t window(int32_t pos) {
-        const int32_t top = (int32_t)b0 + pos - 1;
-        const int32_t a = (top >> 5) + (int32_t)mis;      // ring word index of the window's top word (>= -2 + mis)
-        const uint32_t sh = 31u - ((uint32_t)top & 31u);
-        if ((a >> 2) <= gl + 2) { gl--; fetch(gl); }
+        const int32_t q = pos + qoff;                     // bit index from gbase of the window's top bit (>= -1)
+        const uint32_t o = (uint32_t)q >> 3;              // bits 2-5: ring byte offset of the window's top word
+        const uint32_t sh = ~(uint32_t)q & 31u;
+        if ((q >> 7) <= gl + 2) { gl--; fetch(gl); }
         cp_async_wait_1();
-        const uint32_t h = ring[(uint32_t)a & 15u], m = ring[(uint32_t)(a - 1) & 15u], l = ring[(uint32_t)(a - 2) & 15u];
+        const uint32_t h = word(o), m = word(o - 4u), l = word(o - 8u);
         return ((uint64_t)__funnelshift_l(m, h, sh) << 32) | __funnelshift_l(l, m, sh);
+    }
+    // the ring word at byte offset o mod 64: one LOP3 for the address, since the ring is 64-byte aligned
+    __device__ __forceinline__ uint32_t word(uint32_t o) const {
+#if defined(PNA_EMU)
+        return ring[(o & 60u) >> 2];
+#else
+        uint32_t v;   // volatile: stays behind the cp.async wait that makes the word visible
+        asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(rs | (o & 60u)));
+        return v;
+#endif
     }
 };
 __global__ void __launch_bounds__(32 * SEQ_WARPS) zstd_seq_kernel(const uint8_t* __restrict__ buf, EntryRec* entries, ZBlock* blocks,

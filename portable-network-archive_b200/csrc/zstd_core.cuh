@@ -296,6 +296,8 @@ struct Tab16 {
     uint32_t stride;
     PNA_HD uint32_t get(uint32_t i) const { return p[i * stride]; }
     PNA_HD void set(uint32_t i, uint32_t v) const { p[i * stride] = (uint16_t)v; }
+    // the same table indexed by state + size, the form in which (ns << nbBits) + bits leaves the state
+    PNA_HD Tab16 by_state_plus(uint32_t size) const { return Tab16{p - (size_t)size * stride, stride}; }
 };
 constexpr uint32_t TAB16_LL = 0, TAB16_ML = 512, TAB16_OF = 1024, TAB16_TOTAL = 1280;
 
@@ -432,16 +434,13 @@ PNA_HD uint64_t bits_window(const uint32_t* wb, uint32_t b0, int32_t pos) {
 #endif
     return ((uint64_t)whi << 32) | wlo;
 }
-// n bits (0..32) of window W starting `skip` bits below its top (skip + n <= 64)
-PNA_HD uint32_t win_bits(uint64_t W, uint32_t skip, uint32_t n) {
+// The high word of (hi:lo) << n, 0 <= n <= 31: hi shifted up by n with the top n bits of lo below it.  One SHF on the
+// GPU.  The sequence loop cuts every field with it: (prefix:window) << n appends the window's next n bits to prefix.
+PNA_HD uint32_t shl_hi(uint32_t lo, uint32_t hi, uint32_t n) {
 #if defined(__CUDA_ARCH__)
-    // two 32-bit funnel shifts instead of three emulated 64-bit shifts (this sits on the decode chain)
-    const uint32_t hi = (uint32_t)(W >> 32), lo = (uint32_t)W;
-    const uint32_t a = skip >= 32u ? lo : hi, b = skip >= 32u ? 0u : lo;
-    const uint32_t t = __funnelshift_l(b, a, skip);        // shift taken mod 32: bits [skip, skip + 32) of W
-    return __funnelshift_rc(t, 0u, 32u - n);               // clamped: n == 0 -> 0
+    return __funnelshift_l(lo, hi, n);
 #else
-    return (uint32_t)(((W << skip) >> 1) >> (63 - n));
+    return (uint32_t)(((((uint64_t)hi << 32) | lo) << n) >> 32);
 #endif
 }
 
@@ -469,33 +468,38 @@ struct GlobalBitSrc {
     }
 };
 
-// One block's sequence stream as a stepper, so that a lane can advance several independent streams side by side (the FSE
-// chain of one stream is serial; zstd_seq_kernel interleaves K streams per lane to fill the issue slots its latency leaves).
-// A step is cut in three phases -- call each phase for all of a lane's streams before the next one:
+// One block's sequence stream as a stepper.  A step is cut in three phases:
 //   advance(i)  the loop-carried part: cells -> bit counts -> fields of this sequence, next position, next states
 //   fetch()     the NEXT sequence's bit window and table cells are requested
 //   emit(i)     this sequence's values, repeat-offset logic and the store, in the latency shadow of those loads
+// States are kept as FSE state + table size, which is what (ns << nbBits) + bits gives; the tables are addressed through
+// Tab16::by_state_plus.  Every field is cut from the top of the window with one funnel shift (shl_hi).
 template <class Src>
 struct SeqStream {
     Src src;
     Tab16 tll, tof, tml;
     const uint32_t *llb, *mlb;
     SeqRec* out;
-    uint32_t ulll, ulof, ulml, zll, zof, zml, nseq, lit_regen;
+    uint32_t ulll, ulof, ulml, nseq, lit_regen;
     uint32_t sll, sof, sml, ell, eof, eml;
-    int32_t pos;
+    int32_t pos;       // unread bits; below 0 once the stream is over-read (windows are then read at 0), so end() checks == 0
     uint64_t W;
     uint32_t rep0, rep1, rep2, lit_sum, match_sum, ne, err;
+    // The two per-sequence error tests of the repeat-offset logic, as extremes that end() tests once:
+    //   omin == 0           "rep0 - 1" of an absolute rep0 == 1.  No other offset can be 0, and a symbolic "rep0 - 1"
+    //                       (delta + 1) cannot carry into the slot bits: delta <= nseq < 2^17.
+    //   omax > 2^31 + 2     a new offset (ofv > 3) of 2^31 or more, beyond any legal window.
+    uint32_t omin, omax;
     ZBlock* blk;   // the block's record: escapes (rare) and results go straight there -- the struct holds scalars only, so that
                    // a lane's streams live in registers (an array member would pin them to local memory, which the sequence
                    // kernel's shared-memory carve-out leaves without L1)
     // fields of the sequence between advance() and emit()
-    uint32_t f_ofx, f_x, f_cof, f_xll, f_pll, f_pml;
+    uint32_t f_ofv, f_mlx, f_llx, f_pll, f_pml;
 
     // everything in front of the loop; ST_OK or the status the block fails with
     PNA_HD int32_t begin(const uint32_t* words, const uint8_t* comp, ZBlock& b, const Tab16& tll_, const Tab16& tof_, const Tab16& tml_,
                          int lll, int lof, int lml, const uint32_t* llb_, const uint32_t* mlb_, SeqRec* out_) {
-        tll = tll_; tof = tof_; tml = tml_; llb = llb_; mlb = mlb_; out = out_; blk = &b;
+        llb = llb_; mlb = mlb_; out = out_; blk = &b;
         const uint64_t begin_at = b.src + b.bs_pos;
         const uint32_t len = b.bs_len;
         nseq = b.nseq; lit_regen = b.lit_regen;
@@ -505,68 +509,72 @@ struct SeqStream {
         pos = (int32_t)(len - 1) * 8 + highbit32(last);
         ulll = (uint32_t)lll; ulof = (uint32_t)lof; ulml = (uint32_t)lml;
         if (pos < (int32_t)(ulll + ulof + ulml)) return ST_INVALID_DATA;
+        tll = tll_.by_state_plus(1u << lll); tof = tof_.by_state_plus(1u << lof); tml = tml_.by_state_plus(1u << lml);
         src.init(words, begin_at, pos);
         W = src.window(pos);
-        sll = win_bits(W, 0, ulll); sof = win_bits(W, ulll, ulof); sml = win_bits(W, ulll + ulof, ulml);
+        uint32_t h = (uint32_t)(W >> 32);   // the initial states, <= 9 + 8 + 9 bits: 1 << log prefixes the state's bits
+        sll = shl_hi(h, 1u, ulll); h <<= ulll;
+        sof = shl_hi(h, 1u, ulof); h <<= ulof;
+        sml = shl_hi(h, 1u, ulml);
         pos -= (int32_t)(ulll + ulof + ulml);
         rep0 = REP_SYM | (0u << 29); rep1 = REP_SYM | (1u << 29); rep2 = REP_SYM | (2u << 29);
         lit_sum = 0; match_sum = 0;            // < 2^32: nseq < 2^17 values < 2^17 each
-        zll = 1u << lll; zof = 1u << lof; zml = 1u << lml;
-        ne = 0; err = 0;
+        ne = 0; err = 0; omin = 0xFFFFFFFFu; omax = 0;
         W = src.window(pos);
         ell = tll.get(sll); eof = tof.get(sof); eml = tml.get(sml);
         return ST_OK;
     }
     PNA_HD void advance(uint32_t i) {
-        const uint32_t cll = ell >> 10, cof = eof >> 10, cml = eml >> 10;
-        const uint32_t pll = llb[cll], pml = mlb[cml];       // baseline | extra bits << 24 (seq_pack_base)
+        const uint32_t cof = eof >> 10;
+        const uint32_t pll = llb[ell >> 10], pml = mlb[eml >> 10];   // baseline | extra bits << 24 (seq_pack_ll / _ml)
         const uint32_t xll = pll >> 24, xml = pml >> 24;
         const uint32_t nsl = ell & 1023u, nsm = eml & 1023u, nso = eof & 1023u;
         const uint32_t nbl = ulll - (uint32_t)highbit32(nsl), nbm = ulml - (uint32_t)highbit32(nsm),
                        nbo = ulof - (uint32_t)highbit32(nso);
         const uint32_t xb = cof + xml + xll;                 // value bits: offset, match length, literal length
-        const bool more = i + 1 < nseq;
-        const uint32_t nbs = more ? nbl + nbm + nbo : 0u;    // the last sequence updates no state
-        f_ofx = win_bits(W, 0, cof);
-        f_x = win_bits(W, cof, xml + xll);
-        uint32_t y;
-        if (xb + nbs <= 64u) y = win_bits(W, xb, nbs);
-        else {   // > 64 bits in one sequence (offset codes > 22 with long length codes): second window for the states
+        const uint32_t nbs = i + 1 < nseq ? nbl + nbm + nbo : 0u;   // the last sequence reads no state bits
+        // cut from the top: (h:l) is the window, shifted up past each field as it is taken
+        uint32_t h = (uint32_t)(W >> 32), l = (uint32_t)W;
+        f_ofv = shl_hi(h, 1u, cof);                          // (1 << cof) + cof extra bits
+        h = shl_hi(l, h, cof); l <<= cof;
+        f_mlx = shl_hi(h, 0u, xml);
+        h = shl_hi(l, h, xml); l <<= xml;
+        f_llx = shl_hi(h, 0u, xll);
+        h = shl_hi(l, h, xll);
+        if (xb + nbs > 64u) {   // > 64 bits in one sequence (offset codes > 22 with long length codes): second window for the states
             const int32_t p2 = pos - (int32_t)xb;
-            y = p2 >= 0 ? win_bits(src.window(p2), 0, nbs) : 0u;
+            h = p2 >= 0 ? (uint32_t)(src.window(p2) >> 32) : 0u;
         }
+        // next states (ns << nb) + nb bits, in the order LL, ML, OF; the last sequence's are never used
+        sll = shl_hi(h, nsl, nbl); h <<= nbl;
+        sml = shl_hi(h, nsm, nbm); h <<= nbm;
+        sof = shl_hi(h, nso, nbo);
         pos -= (int32_t)(xb + nbs);
-        err |= (uint32_t)(pos < 0);
-        pos = pos < 0 ? 0 : pos;                             // keep the reads inside the arena on corrupt input
-        sll = more ? ((nsl << nbl) - zll) + (y >> (nbm + nbo)) : 0u;
-        sml = more ? ((nsm << nbm) - zml) + ((y >> nbo) & ((1u << nbm) - 1u)) : 0u;
-        sof = more ? ((nso << nbo) - zof) + (y & ((1u << nbo) - 1u)) : 0u;
-        f_cof = cof; f_xll = xll; f_pll = pll; f_pml = pml;
+        f_pll = pll; f_pml = pml;
     }
-    PNA_HD void fetch() {   // (after the last sequence: position 0 / state 0, valid and unused)
-        W = src.window(pos);
+    PNA_HD void fetch() {
+        W = src.window(pos < 0 ? 0 : pos);                   // keep the reads inside the arena on corrupt input
         ell = tll.get(sll); eof = tof.get(sof); eml = tml.get(sml);
     }
     PNA_HD void emit(uint32_t i) {
-        const uint32_t mlx = f_x >> f_xll, llx = f_x & ((1u << f_xll) - 1u);
-        const uint32_t ofv = (1u << f_cof) + f_ofx;
-        const uint32_t ml = (f_pml & 0xFFFFFFu) + mlx;
-        const uint32_t ll = (f_pll & 0xFFFFFFu) + llx;
-        // repeat-offset logic (RFC 8878 3.1.1.5), branch-free; offsets may be symbolic (REP_SYM) in the block's incoming history
-        const bool is_new = ofv > 3;
-        const uint32_t idx = ofv - 1 + (ll == 0 ? 1u : 0u);                     // meaningful when !is_new: 0..3
-        const uint32_t dec = (rep0 & REP_SYM) ? rep0 + 1 : rep0 - 1;            // "rep0 - 1" (symbolic: delta + 1)
-        const uint32_t cand = idx == 0 ? rep0 : idx == 1 ? rep1 : idx == 2 ? rep2 : dec;
-        const uint32_t off = is_new ? ofv - 3 : cand;
-        err |= (uint32_t)(is_new && (off & REP_SYM) != 0);
-        err |= (uint32_t)(!is_new && idx == 3 && ((rep0 & REP_SYM) ? (off & 0x1FFFFFFFu) == 0 : off == 0));
-        const bool sh2 = is_new || idx >= 2, sh1 = is_new || idx >= 1;
-        rep2 = sh2 ? rep1 : rep2;
-        rep1 = sh1 ? rep0 : rep1;
+        const uint32_t ml = (f_pml & 0xFFFFFFu) + f_mlx;
+        const uint32_t ll = (f_pll & 0xFFFFFFu) + f_llx;
+        const uint32_t ofv = f_ofv;
+        // repeat-offset logic (RFC 8878 3.1.1.5), branch-free; offsets may be symbolic (REP_SYM) in the block's incoming history.
+        // idx 0..2 picks rep0..rep2; idx >= 3 is a new offset (ofv > 3) or "rep0 - 1" (ofv == 3 with ll == 0)
+        const uint32_t idx = ofv - (ll < 1u ? ll : 1u);
+        const uint32_t dec = rep0 - 1u + ((rep0 >> 30) & 2u);     // "rep0 - 1" (symbolic: delta + 1)
+        const uint32_t nw = ofv == 3u ? dec : ofv - 3u;
+        const uint32_t r12 = idx >= 2u ? rep2 : rep1;
+        const uint32_t off = idx >= 3u ? nw : idx >= 1u ? r12 : rep0;
+        omin = off < omin ? off : omin;
+        omax = ofv > omax ? ofv : omax;
+        rep2 = idx >= 2u ? rep1 : rep2;
+        rep1 = idx >= 1u ? rep0 : rep1;
         rep0 = off;
         SeqRec r;
         r.x = off;
-        r.y = ll | (ml << 16);
+        r.y = ll + (ml << 16);
         if ((ll | ml) >= SEQ_ESC) {                          // cheap superset of "a length does not fit 16 bits" (rare)
             if (ll >= SEQ_ESC || ml >= SEQ_ESC) {
                 if (ne < (uint32_t)SEQ_ESC_MAX) { blk->esc_idx[ne] = i; blk->esc_ll[ne] = ll; blk->esc_ml[ne] = ml; }
@@ -575,13 +583,17 @@ struct SeqStream {
             }
             r.y = (ll < SEQ_ESC ? ll : SEQ_ESC) | ((ml < SEQ_ESC ? ml : SEQ_ESC) << 16);
         }
-        out[i] = r;
+#if defined(__CUDA_ARCH__)
+        *reinterpret_cast<uint2*>(out++) = make_uint2(r.x, r.y);   // one 8-byte store (records are 8-byte aligned)
+#else
+        *out++ = r;
+#endif
         lit_sum += ll; match_sum += ml;
     }
     PNA_HD void step(uint32_t i) { advance(i); fetch(); emit(i); }
     // after the last sequence: final checks, block totals, outgoing history, escapes
     PNA_HD int32_t end() {
-        if (err || pos != 0) return ST_INVALID_DATA;
+        if (err || pos != 0 || omin == 0 || omax > 0x80000002u) return ST_INVALID_DATA;
         if (lit_sum > lit_regen) return ST_INVALID_DATA;
         const uint64_t outsz = (uint64_t)lit_regen + match_sum;
         if (outsz > BLOCK_MAX) return ST_INVALID_DATA;

@@ -21,7 +21,7 @@
 // (or far matches > FAR_MAX bytes) go one at a time through whole-CTA copies.
 //
 // Two instantiations: LzSmall (4 warps, 16-bit codes, 29 KB of shared memory: 7 CTAs = 28 warps per SM, one wave
-// for 1024 entries on 148 SMs) and LzBig (32 warps, 32-bit codes, 128 KiB window) for batches with fewer entries
+// for 1024 entries on 148 SMs) and LzBig (16 warps, 32-bit codes, 128 KiB window) for batches with fewer entries
 // than SMs -- a solid archive is ONE frame.
 #pragma once
 #include <cuda_runtime.h>

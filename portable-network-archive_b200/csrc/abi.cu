@@ -195,55 +195,48 @@ static const CipherKernel<decltype(&decrypt_tiles_kernel<0, 1>)> DECRYPT_TILES[4
     {decrypt_tiles_kernel<2, 0>, CAM_SMEM}};      // Camellia-CBC
 constexpr int ECB_SMEM = AES_DEC_SMEM;
 
-namespace pna { namespace multi {
-// LPT: heaviest entries first onto the least loaded device; each device keeps its entries in caller order
-static std::vector<std::vector<uint32_t>> shard(const std::vector<uint64_t>& weight, size_t n_dev) {
-    std::vector<uint32_t> order(weight.size());
-    for (uint32_t i = 0; i < order.size(); i++) order[i] = i;
-    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return weight[a] > weight[b]; });
-    std::vector<uint64_t> load(n_dev, 0);
-    std::vector<std::vector<uint32_t>> part(n_dev);
-    for (uint32_t i : order) {
-        size_t best = 0;
-        for (size_t d = 1; d < n_dev; d++) if (load[d] < load[best]) best = d;
-        part[best].push_back(i);
-        load[best] += weight[i] + 1;
+// Expanded key schedule of one (cipher, key): encryption 1 AES-256, 2 Camellia-256
+static DevKeys expand_key(const pna_ctx* ctx, uint8_t encryption, const uint8_t key[32]) {
+    DevKeys dk;
+    memset(&dk, 0, sizeof dk);
+    if (encryption == 1) {
+        AesKey ak; aes256_expand_key(&ctx->h_aes, key, &ak);
+        memcpy(dk.aes_rk, ak.rk, sizeof ak.rk); memcpy(dk.aes_dk, ak.dk, sizeof ak.dk);
+    } else {
+        CamelliaKey ck; camellia256_expand_key(&ctx->h_cam, key, &ck);
+        memcpy(dk.cam_ek, ck.ek, sizeof ck.ek); memcpy(dk.cam_dk, ck.dk, sizeof ck.dk);
     }
-    for (auto& p : part) std::sort(p.begin(), p.end());
-    return part;
+    return dk;
 }
-// f(d) on one host thread per device; the first non-zero return code wins
-template <class F>
-static int for_devices(size_t n_dev, F&& f) {
-    std::vector<int> rc(n_dev, PNA_OK);
-    std::vector<std::thread> th;
-    for (size_t d = 1; d < n_dev; d++) th.emplace_back([&, d]() { rc[d] = f(d); });
-    rc[0] = f(0);
-    for (auto& t : th) t.join();
-    for (int r : rc) if (r != PNA_OK) return r;
-    return PNA_OK;
-}
-static void carry_error(pna_ctx* root) {
-    for (pna_ctx* c : root->devs) if (!c->err.empty()) { root->err = "device " + std::to_string(c->device) + ": " + c->err; return; }
-}
+// The key schedules of one plan, one per distinct (cipher, key); entries refer to them by index
+struct KeyTable {
+    std::vector<DevKeys> keys;
+    std::map<std::array<uint8_t, 33>, int> ids;
+    int index(const pna_ctx* ctx, uint8_t encryption, const uint8_t key[32]) {
+        std::array<uint8_t, 33> k;
+        k[0] = encryption;
+        memcpy(k.data() + 1, key, 32);
+        auto it = ids.find(k);
+        if (it == ids.end()) {
+            it = ids.emplace(k, (int)keys.size()).first;
+            keys.push_back(expand_key(ctx, encryption, key));
+        }
+        return it->second;
+    }
+};
 
-static int crc32(pna_ctx* root, const pna_span* spans, uint32_t n, uint32_t* crc_out);
-static int decode_plan_create(pna_ctx* root, const pna_decode_desc* descs, uint32_t n, const uint8_t* image, uint64_t image_len,
-                              const pna_span* crc_spans, const uint32_t* crc_expect, const int32_t* crc_entry, uint32_t n_spans, bool with_crc,
-                              pna_plan** plan);
-static int decode_plan_run(pna_plan* P);
-static int decode_plan_fetch(pna_plan* P, pna_buf* out, int32_t* status);
-static int decode_plan_lengths(pna_plan* P, uint64_t* out_len, int32_t* status);
-static int plan_crc_results(pna_plan* P, uint32_t* crc_out, uint32_t* n_broken);
-static void plan_destroy(pna_plan* P);
-static int encode_plan_create(pna_ctx* root, const pna_encode_desc* descs, uint32_t n, pna_plan** plan);
-static int encode_plan_run(pna_plan* P);
-static int encode_plan_lengths(pna_plan* P, uint64_t* out_len, int32_t* status);
-static int encode_plan_fetch(pna_plan* P, pna_buf* out, uint32_t* fdat_crc_out, uint32_t* crc_count_out, int32_t* status);
-static int route(pna_plan* P, uint32_t entry, pna_plan** sub, uint32_t* local);
-static void sum_stats(pna_plan* P, uint64_t* a, uint64_t* b, uint64_t* c, bool counts);
-static int stage_ms(pna_plan* P, float* ms, uint32_t cap);
-}}
+// The reference's dispatch on an entry's compression, encryption and cipher mode (entry/read.rs:59-190): ST_UNSUPPORTED
+// for a value it does not know, else ST_OK.  Decode and encode accept the same set.
+static int32_t entry_mode_status(uint8_t compression, uint8_t encryption, uint8_t cipher_mode) {
+    if (compression != PNA_COMPRESSION_NO && compression != PNA_COMPRESSION_DEFLATE && compression != PNA_COMPRESSION_ZSTD &&
+        compression != PNA_COMPRESSION_XZ)
+        return ST_UNSUPPORTED;
+    if (encryption != PNA_ENCRYPTION_NO && encryption != PNA_ENCRYPTION_AES && encryption != PNA_ENCRYPTION_CAMELLIA)
+        return ST_UNSUPPORTED;
+    if (encryption != 0 && cipher_mode != PNA_CIPHER_CBC && cipher_mode != PNA_CIPHER_CTR && cipher_mode != PNA_CIPHER_GCM)
+        return ST_UNSUPPORTED;
+    return ST_OK;
+}
 
 // ------------------------------------------------------------------------------------------------
 // Host span -> device image staging with range coalescing: spans that lie close together in host
@@ -309,11 +302,13 @@ struct GcmDev {
     uint32_t n_segs = 0, n_tiles = 0, n_tiles_aes = 0, n_keys = 0;
 };
 
+// chunk-CRC spans a decode plan verifies on its uploaded image (pna_cuda_decode_plan_create_crc / _in_image)
+struct CrcReq { const pna_span* spans; const uint32_t* expect; const int32_t* entry_of; uint32_t n; const uint8_t* image; uint64_t image_len; };
+
 namespace pna { namespace multi { struct Plan; } }
 // ------------------------------------------------------------------------------------------------
 struct pna_plan {
     pna::multi::Plan* multi = nullptr;   // set: a plan of a multi-device context (multi_host.cuh); everything below is unused then
-    std::vector<uint64_t> h_crc_count_bound;
     pna_ctx* ctx = nullptr;
     int kind = 0;   // 0 decode, 1 encode
     uint32_t n = 0;
@@ -322,7 +317,7 @@ struct pna_plan {
     // host metadata
     std::vector<EntryRec> h_entries;
     std::vector<Segment> h_segs;
-    std::vector<DevKeys> h_keys;
+    KeyTable h_keys;
     std::vector<CipherTile> h_tiles[4];   // by variant_of: 0 gather, 1 aes-cbc, 2 camellia-ctr, 3 camellia-cbc
     std::vector<CtrTile> h_ctr_tiles;     // aes-ctr
     std::vector<uint32_t> h_store, h_deflate, h_xz;
@@ -398,6 +393,8 @@ struct pna_plan {
         if (enc) enc::destroy(enc);
     }
 };
+
+#include "multi_host.cuh"
 
 // ------------------------------------------------------------------------------------------------
 extern "C" const char* pna_cuda_strerror(int32_t s) {
@@ -578,20 +575,22 @@ static int launch_chunk_crc(pna_ctx* ctx, const uint8_t* img, const CrcTile* til
     LAUNCHED();
     return PNA_OK;
 }
+// the next span (l bytes at device offset o): its first tile into `first`, its CRC_TILE tiles (one, empty, for l == 0) into `tiles`
+static void add_crc_span(std::vector<CrcTile>& tiles, std::vector<uint32_t>& first, uint64_t o, uint64_t l) {
+    const uint32_t i = (uint32_t)first.size();
+    first.push_back((uint32_t)tiles.size());
+    do {
+        uint32_t t = (uint32_t)std::min<uint64_t>(l, CRC_TILE);
+        tiles.push_back({o, t, i});
+        o += t; l -= t;
+    } while (l);
+}
 static int crc_run(pna_ctx* ctx, const uint8_t* d_img, const std::vector<uint64_t>& off, const uint64_t* len, uint32_t n,
                    uint32_t* crc_out) {
     std::vector<CrcTile> tiles;
-    std::vector<uint32_t> first(n);
-    tiles.reserve(n);
-    for (uint32_t i = 0; i < n; i++) {
-        first[i] = (uint32_t)tiles.size();
-        uint64_t o = off[i], l = len[i];
-        do {
-            uint32_t t = (uint32_t)std::min<uint64_t>(l, CRC_TILE);
-            tiles.push_back({o, t, i});
-            o += t; l -= t;
-        } while (l);
-    }
+    std::vector<uint32_t> first;
+    tiles.reserve(n); first.reserve(n);
+    for (uint32_t i = 0; i < n; i++) add_crc_span(tiles, first, off[i], len[i]);
     const uint32_t nt = (uint32_t)tiles.size();
     DevArr<CrcTile> d_tiles; DevArr<uint32_t> d_first, d_raw, d_crc;
     CK(d_tiles.upload(tiles, ctx->stream)); CK(d_first.upload(first, ctx->stream));
@@ -626,11 +625,7 @@ extern "C" int pna_cuda_crc32_image(pna_ctx* ctx, const uint8_t* image, uint64_t
     if (n == 0) return PNA_OK;
     for (uint32_t i = 0; i < n; i++)
         if (span_off[i] > image_len || span_len[i] > image_len - span_off[i]) return PNA_E_BAD_ARG;
-    if (!ctx->devs.empty()) {
-        std::vector<pna_span> sp(n);
-        for (uint32_t i = 0; i < n; i++) sp[i] = {image + span_off[i], span_len[i]};
-        return multi::crc32(ctx, sp.data(), n, crc_out);
-    }
+    if (!ctx->devs.empty()) return multi::crc32_image(ctx, image, span_off, span_len, n, crc_out);
     std::lock_guard<std::mutex> g(ctx->mu);
     CK(cudaSetDevice(ctx->device));
     DevArr<uint8_t> d_img;
@@ -667,7 +662,6 @@ static bool size_hint_trusted(uint8_t compression, uint64_t comp_len, uint64_t h
     return !(hint > ((uint64_t)1 << 30) && hint / 256 > comp_len);   // huge both absolutely and relative to the stream
 }
 extern "C" int pna_cuda_size_hint_trusted(uint8_t compression, uint64_t stream_len, uint64_t hint) { return size_hint_trusted(compression, stream_len, hint) ? 1 : 0; }
-struct CrcReq { const pna_span* spans; const uint32_t* expect; const int32_t* entry_of; uint32_t n; const uint8_t* image; uint64_t image_len; };
 // AES-CTR tiles of entry i (aes_ctr_tiles_kernel): cut at body boundaries and after CTR_TILE_RUNS counter runs; a block that
 // straddles two bodies becomes a one-block tile gathered through the segments.  The IV is read here, from the host bodies.
 static void ctr_tiles(pna_plan* P, const pna_decode_desc& d, uint32_t i) {
@@ -733,7 +727,6 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
         }
         st.sealed = true;   // bodies now only look up / extend; see Stager::add
     }
-    std::map<std::array<uint8_t, 33>, int> key_ids;
     uint64_t comp_extra = 0;   // bytes needed in the comp region (decrypted / gathered streams)
     std::vector<uint8_t> needs_copy(n, 0);
     std::vector<gcm::GcmSeg> gcm_walk;            // segments in entry order
@@ -756,14 +749,9 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
         e.stream_len = pos;
         P->stream_bytes += pos;
         // host-side validation == the reference's dispatch (entry/read.rs:59-190)
-        if (d.compression != PNA_COMPRESSION_NO && d.compression != PNA_COMPRESSION_DEFLATE && d.compression != PNA_COMPRESSION_ZSTD &&
-            d.compression != PNA_COMPRESSION_XZ)
-            e.status = ST_UNSUPPORTED;
-        else if (d.encryption != PNA_ENCRYPTION_NO && d.encryption != PNA_ENCRYPTION_AES && d.encryption != PNA_ENCRYPTION_CAMELLIA)
-            e.status = ST_UNSUPPORTED;
-        else if (d.encryption != 0 && d.cipher_mode != PNA_CIPHER_CBC && d.cipher_mode != PNA_CIPHER_CTR && d.cipher_mode != PNA_CIPHER_GCM)
-            e.status = ST_UNSUPPORTED;
-        else if (d.encryption != 0 && d.cipher_mode == PNA_CIPHER_GCM) {
+        e.status = entry_mode_status(d.compression, d.encryption, d.cipher_mode);
+        if (e.status != ST_OK) continue;
+        if (d.encryption != 0 && d.cipher_mode == PNA_CIPHER_GCM) {
             // stream header + segment walk (entry/read.rs:105-118, aead.rs:134-148, gcm.rs:206-262); every layout violation
             // is an AeadError == InvalidData (error.rs:67-74)
             uint8_t hdr[gcm::GCM_HEADER_LEN];
@@ -805,24 +793,7 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
             e.status = ST_UNEXPECTED_EOF;   // cipher/block/read.rs:36,90
         if (e.status != ST_OK) continue;
         if (d.encryption) {
-            std::array<uint8_t, 33> k;
-            k[0] = d.encryption;
-            memcpy(k.data() + 1, d.key, 32);
-            auto it = key_ids.find(k);
-            if (it == key_ids.end()) {
-                DevKeys dk;
-                memset(&dk, 0, sizeof dk);
-                if (d.encryption == 1) {
-                    AesKey ak; aes256_expand_key(&ctx->h_aes, d.key, &ak);
-                    memcpy(dk.aes_rk, ak.rk, sizeof ak.rk); memcpy(dk.aes_dk, ak.dk, sizeof ak.dk);
-                } else {
-                    CamelliaKey ck; camellia256_expand_key(&ctx->h_cam, d.key, &ck);
-                    memcpy(dk.cam_ek, ck.ek, sizeof ck.ek); memcpy(dk.cam_dk, ck.dk, sizeof ck.dk);
-                }
-                it = key_ids.emplace(k, (int)P->h_keys.size()).first;
-                P->h_keys.push_back(dk);
-            }
-            e.key_idx = it->second;
+            e.key_idx = P->h_keys.index(ctx, d.encryption, d.key);
             e.comp_len = d.cipher_mode == PNA_CIPHER_GCM ? gcm_len[i] : pos - 16;   // CBC: rewritten by the kernel after unpadding
             needs_copy[i] = 1;
         } else {
@@ -833,18 +804,9 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
     }
     P->image_bytes = align_up(st.total, 256);
     if (P->n_crc) {
-        P->h_crc_first.resize(P->n_crc);
         P->h_crc_expect.assign(crc->expect, crc->expect + crc->n);
         P->h_crc_entry.assign(crc->entry_of, crc->entry_of + crc->n);
-        for (uint32_t i = 0; i < P->n_crc; i++) {
-            P->h_crc_first[i] = (uint32_t)P->h_crc_tiles.size();
-            uint64_t o = crc_off[i], l = crc->spans[i].len;
-            do {
-                uint32_t t = (uint32_t)std::min<uint64_t>(l, CRC_TILE);
-                P->h_crc_tiles.push_back({o, t, i});
-                o += t; l -= t;
-            } while (l);
-        }
+        for (uint32_t i = 0; i < P->n_crc; i++) add_crc_span(P->h_crc_tiles, P->h_crc_first, crc_off[i], crc->spans[i].len);
     }
     // comp region right behind the image
     uint64_t cur = P->image_bytes;
@@ -924,11 +886,11 @@ static int decode_plan_build(pna_ctx* ctx, const pna_decode_desc* descs, uint32_
     CK(P->d_buf.reserve(P->buf_bytes));
     CK(P->d_entries.reserve(n)); CK(P->d_entries_init.reserve(n));
     CK(P->d_segs.reserve(P->h_segs.size()));
-    CK(P->d_keys.reserve(P->h_keys.size()));
+    CK(P->d_keys.reserve(P->h_keys.keys.size()));
     int rc = st.upload(ctx, P->d_buf.p);
     if (rc) return rc;
     cudaStream_t s = ctx->stream;
-    CK(P->d_segs.upload(P->h_segs, s)); CK(P->d_keys.upload(P->h_keys, s));
+    CK(P->d_segs.upload(P->h_segs, s)); CK(P->d_keys.upload(P->h_keys.keys, s));
     CK(P->d_ctr_tiles.upload(P->h_ctr_tiles, s));
     for (int v = 0; v < 4; v++) CK(P->d_tiles[v].upload(P->h_tiles[v], s));
     CK(P->d_deflate.upload(P->h_deflate, s)); CK(P->d_xz.upload(P->h_xz, s));
@@ -1389,12 +1351,6 @@ static int decode_launch_all(pna_plan* P, bool fresh) {
         if ((rc = launch_cipher(P))) return rc;
         STAGE(2);
         if ((rc = launch_zstd_front(P, false))) return rc;
-        STAGE(3);
-        if ((rc = launch_zstd_seq(P))) return rc;
-        STAGE(4);
-        if ((rc = launch_zstd_lit(P))) return rc;
-        STAGE(5);
-        if ((rc = launch_zstd_prefix(P))) return rc;
     } else {
         std::vector<uint64_t> oc(2 * (size_t)P->n);
         for (uint32_t i = 0; i < P->n; i++) { oc[2 * i] = P->h_entries[i].out_off; oc[2 * i + 1] = P->h_entries[i].out_cap; }
@@ -1402,15 +1358,15 @@ static int decode_launch_all(pna_plan* P, bool fresh) {
         set_layout_kernel<<<(P->n + 127) / 128, 128, 0, ctx->stream>>>(P->d_entries.p, P->d_layout.p, P->n);
         LAUNCHED();
         CK(ctx->sync());   // oc is a local
-        STAGE(0); STAGE(1); STAGE(2); STAGE(3);
-        if (!P->sized_entropy) {
-            if ((rc = launch_zstd_seq(P))) return rc;
-            STAGE(4);
-            if ((rc = launch_zstd_lit(P))) return rc;
-            STAGE(5);
-            if ((rc = launch_zstd_prefix(P))) return rc;
-        } else { STAGE(4); STAGE(5); }
+        STAGE(0); STAGE(1); STAGE(2);
     }
+    STAGE(3);
+    const bool entropy = fresh || !P->sized_entropy;   // decode_prepare's sizing pass leaves the entropy stages done
+    if (entropy && (rc = launch_zstd_seq(P))) return rc;
+    STAGE(4);
+    if (entropy && (rc = launch_zstd_lit(P))) return rc;
+    STAGE(5);
+    if (entropy && (rc = launch_zstd_prefix(P))) return rc;
     STAGE(6);
     if ((rc = launch_zstd_lz(P))) return rc;
     STAGE(7);
@@ -1427,9 +1383,7 @@ static int decode_plan_create_ex(pna_ctx* ctx, const pna_decode_desc* descs, uin
                                  pna_plan** plan) {
     if (!ctx || !plan || (!descs && n)) return PNA_E_BAD_ARG;
     *plan = nullptr;
-    if (!ctx->devs.empty())   // (caps only come from pna_cuda_decode_batch, which shards before it gets here)
-        return multi::decode_plan_create(ctx, descs, n, crc ? crc->image : nullptr, crc ? crc->image_len : 0, crc ? crc->spans : nullptr,
-                                         crc ? crc->expect : nullptr, crc ? crc->entry_of : nullptr, crc ? crc->n : 0, crc != nullptr, plan);
+    if (!ctx->devs.empty()) return multi::decode_plan_create(ctx, descs, n, crc, plan);   // (caps only come from pna_cuda_decode_batch, which shards first)
     std::lock_guard<std::mutex> g(ctx->mu);
     CK(cudaSetDevice(ctx->device));
     pna_plan* P = new pna_plan();
@@ -1485,6 +1439,16 @@ extern "C" int pna_cuda_decode_plan_run(pna_plan* P) {
     }
     return decode_launch_all(P, true);
 }
+// An entry's status and decoded length after a run, from its host record `h` and its device record `d`: a host-side
+// rejection first, then the device's status, then the plan's capacity.  The length is 0 unless the status is OK or NOSPACE.
+static int32_t decode_result(const EntryRec& h, const EntryRec& d, uint64_t* len) {
+    int32_t st = d.status;
+    uint64_t l = d.compression == PNA_COMPRESSION_NO ? d.comp_len : d.out_len;
+    if (h.status != ST_OK) { st = h.status; l = 0; }
+    if (st == ST_OK && l > d.out_cap) st = ST_NOSPACE;
+    *len = (st == ST_OK || st == ST_NOSPACE) ? l : 0;
+    return st;
+}
 extern "C" int pna_cuda_decode_plan_fetch(pna_plan* P, pna_buf* out, int32_t* status) {
     if (!P || P->kind != 0 || ((!out || !status) && P->n)) return PNA_E_BAD_ARG;
     if (P->multi) return multi::decode_plan_fetch(P, out, status);
@@ -1509,12 +1473,10 @@ extern "C" int pna_cuda_decode_plan_fetch(pna_plan* P, pna_buf* out, int32_t* st
     uint32_t prev = UINT32_MAX;
     for (uint32_t i = 0; i < P->n; i++) {
         const EntryRec& e = dev[i];
-        int32_t st = e.status;
-        uint64_t len = e.compression == PNA_COMPRESSION_NO ? e.comp_len : e.out_len;
-        if (P->h_entries[i].status != ST_OK) { st = P->h_entries[i].status; len = 0; }
-        if (st == ST_OK && len > e.out_cap) st = ST_NOSPACE;
+        uint64_t len;
+        int32_t st = decode_result(P->h_entries[i], e, &len);
         if (st == ST_OK && len > out[i].cap) st = ST_NOSPACE;
-        out[i].len = (st == ST_OK || st == ST_NOSPACE) ? len : 0;
+        out[i].len = len;
         status[i] = st;
         if (st == ST_OK && len) {
             bool merged = false;
@@ -1554,16 +1516,10 @@ extern "C" int pna_cuda_decode_plan_lengths(pna_plan* P, uint64_t* out_len, int3
     std::vector<EntryRec> dev(P->n);
     CK(cudaMemcpyAsync(dev.data(), P->d_entries.p, P->n * sizeof(EntryRec), cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx->sync());
-    P->h_out_len.assign(P->n, 0);
+    P->h_out_len.resize(P->n);
     for (uint32_t i = 0; i < P->n; i++) {
-        const EntryRec& e = dev[i];
-        int32_t st = e.status;
-        uint64_t len = e.compression == PNA_COMPRESSION_NO ? e.comp_len : e.out_len;
-        if (P->h_entries[i].status != ST_OK) { st = P->h_entries[i].status; len = 0; }
-        if (st == ST_OK && len > e.out_cap) st = ST_NOSPACE;
-        out_len[i] = (st == ST_OK || st == ST_NOSPACE) ? len : 0;
-        status[i] = st;
-        if (st == ST_OK) P->h_out_len[i] = len;
+        status[i] = decode_result(P->h_entries[i], dev[i], &out_len[i]);
+        P->h_out_len[i] = status[i] == ST_OK ? out_len[i] : 0;
     }
     return PNA_OK;
 }
@@ -1576,11 +1532,7 @@ static int plan_entry_out(pna_plan* P, uint32_t entry, const uint8_t** base, uin
 }
 extern "C" int pna_cuda_decode_plan_crc32_out(pna_plan* P, uint32_t entry, const uint64_t* span_off, const uint64_t* span_len,
                                               uint32_t n, uint32_t* crc_out) {
-    if (P && P->multi) {
-        pna_plan* sub = nullptr; uint32_t loc = 0;
-        const int r = multi::route(P, entry, &sub, &loc);
-        return r ? r : pna_cuda_decode_plan_crc32_out(sub, loc, span_off, span_len, n, crc_out);
-    }
+    if (P && P->multi) P = multi::route(P, &entry);
     const uint8_t* base = nullptr;
     uint64_t len = 0;
     int rc = plan_entry_out(P, entry, &base, &len);
@@ -1596,11 +1548,7 @@ extern "C" int pna_cuda_decode_plan_crc32_out(pna_plan* P, uint32_t entry, const
 }
 extern "C" int pna_cuda_decode_plan_fetch_ranges(pna_plan* P, uint32_t entry, const uint64_t* src_off, const uint64_t* len,
                                                  uint8_t* const* dst, uint32_t n) {
-    if (P && P->multi) {
-        pna_plan* sub = nullptr; uint32_t loc = 0;
-        const int r = multi::route(P, entry, &sub, &loc);
-        return r ? r : pna_cuda_decode_plan_fetch_ranges(sub, loc, src_off, len, dst, n);
-    }
+    if (P && P->multi) P = multi::route(P, &entry);
     const uint8_t* base = nullptr;
     uint64_t total = 0;
     int rc = plan_entry_out(P, entry, &base, &total);
@@ -1667,24 +1615,7 @@ extern "C" void pna_cuda_plan_destroy(pna_plan* P) {
 extern "C" int pna_cuda_decode_batch(pna_ctx* ctx, const pna_decode_desc* descs, uint32_t n, pna_buf* out, int32_t* status) {
     if (!ctx || ((!descs || !out || !status) && n)) return PNA_E_BAD_ARG;
     if (n == 0) return PNA_OK;
-    if (!ctx->devs.empty()) {   // shard by entry, one ordinary batch per device
-        std::vector<uint64_t> w(n);
-        for (uint32_t i = 0; i < n; i++) { uint64_t b = 0; for (uint32_t k = 0; k < descs[i].n_bodies; k++) b += descs[i].bodies[k].len; w[i] = b; }
-        const auto part = multi::shard(w, ctx->devs.size());
-        const int rc = multi::for_devices(ctx->devs.size(), [&](size_t d) -> int {
-            const auto& idx = part[d];
-            if (idx.empty()) return PNA_OK;
-            std::vector<pna_decode_desc> dd(idx.size());
-            std::vector<pna_buf> bb(idx.size());
-            std::vector<int32_t> st(idx.size());
-            for (size_t k = 0; k < idx.size(); k++) { dd[k] = descs[idx[k]]; bb[k] = out[idx[k]]; }
-            const int r = pna_cuda_decode_batch(ctx->devs[d], dd.data(), (uint32_t)dd.size(), bb.data(), st.data());
-            if (r == PNA_OK) for (size_t k = 0; k < idx.size(); k++) { out[idx[k]].len = bb[k].len; status[idx[k]] = st[k]; }
-            return r;
-        });
-        if (rc) multi::carry_error(ctx);
-        return rc;
-    }
+    if (!ctx->devs.empty()) return multi::decode_batch(ctx, descs, n, out, status);
     std::vector<uint64_t> caps(n);
     for (uint32_t i = 0; i < n; i++) caps[i] = out[i].cap;
     pna_plan* P = nullptr;
@@ -1735,15 +1666,7 @@ extern "C" int pna_cuda_ecb(pna_ctx* ctx, int encryption, int encrypt, const uin
     if (!nb) return PNA_OK;
     std::lock_guard<std::mutex> g(ctx->mu);
     CK(cudaSetDevice(ctx->device));
-    DevKeys dk;
-    memset(&dk, 0, sizeof dk);
-    if (encryption == 1) {
-        AesKey ak; aes256_expand_key(&ctx->h_aes, key, &ak);
-        memcpy(dk.aes_rk, ak.rk, sizeof ak.rk); memcpy(dk.aes_dk, ak.dk, sizeof ak.dk);
-    } else {
-        CamelliaKey ck; camellia256_expand_key(&ctx->h_cam, key, &ck);
-        memcpy(dk.cam_ek, ck.ek, sizeof ck.ek); memcpy(dk.cam_dk, ck.dk, sizeof ck.dk);
-    }
+    const DevKeys dk = expand_key(ctx, (uint8_t)encryption, key);
     DevArr<uint8_t> d_in, d_out; DevArr<DevKeys> d_key;
     CK(d_in.reserve(nb * 16 + 64)); CK(d_out.reserve(nb * 16));
     CK(cudaMemcpyAsync(d_in.p, in, nb * 16, cudaMemcpyHostToDevice, ctx->stream));
@@ -1759,4 +1682,3 @@ extern "C" int pna_cuda_ecb(pna_ctx* ctx, int encryption, int encrypt, const uin
 // ------------------------------------------------------------------------------------------------
 // seam 3: encode -- implemented in encode_host.cuh on top of kernels_encode.cuh
 #include "encode_host.cuh"
-#include "multi_host.cuh"

@@ -6,7 +6,7 @@ namespace pna { namespace enc {
 struct EncodePlan {
     std::vector<EncEntry> h_entries;
     std::vector<SegRec> h_segs;
-    std::vector<DevKeys> h_keys;
+    KeyTable h_keys;
     std::vector<CipherTile> h_tiles[3];       // 0 none (gather), 1 aes-ctr, 2 camellia-ctr
     std::vector<uint32_t> h_cbc[2];           // aes, camellia
     std::vector<CrcTileSrc> h_crc_src;
@@ -90,7 +90,6 @@ static int encode_plan_build(pna_ctx* ctx, const pna_encode_desc* descs, uint32_
     EncodePlan* E = new EncodePlan();
     P->enc = E;
     E->h_entries.resize(n);
-    std::map<std::array<uint8_t, 33>, int> key_ids;
     // work arena: [plain | literals (same layout) | per-segment tmp | per-entry header scratch]
     uint64_t plain_total = 0, nsegs_total = 0;
     for (uint32_t i = 0; i < n; i++) {
@@ -107,38 +106,13 @@ static int encode_plan_build(pna_ctx* ctx, const pna_encode_desc* descs, uint32_
         if (d.compression == PNA_COMPRESSION_XZ) E->has_xz[enc::xz_lc_for_effort(e.effort)] = true;
         memcpy(e.iv, d.iv, 16);
         e.key_idx = -1;
-        if (d.compression != PNA_COMPRESSION_NO && d.compression != PNA_COMPRESSION_DEFLATE && d.compression != PNA_COMPRESSION_ZSTD &&
-            d.compression != PNA_COMPRESSION_XZ)
-            e.status = ST_UNSUPPORTED;
-        else if (d.encryption != PNA_ENCRYPTION_NO && d.encryption != PNA_ENCRYPTION_AES && d.encryption != PNA_ENCRYPTION_CAMELLIA)
-            e.status = ST_UNSUPPORTED;
-        else if (d.encryption != 0 && d.cipher_mode != PNA_CIPHER_CBC && d.cipher_mode != PNA_CIPHER_CTR && d.cipher_mode != PNA_CIPHER_GCM)
-            e.status = ST_UNSUPPORTED;
-        else if (enc_is_gcm(d) && enc_gcm_seg_size(d) == 0)
+        e.status = entry_mode_status(d.compression, d.encryption, d.cipher_mode);
+        if (e.status == ST_OK && enc_is_gcm(d) && enc_gcm_seg_size(d) == 0)
             e.status = ST_INVALID_INPUT;   // no stream header / segment size out of range (SegmentSize::new, aead.rs:83-88)
         if (e.status != ST_OK) continue;
         if (enc_is_gcm(d)) { e.gcm_seg_size = enc_gcm_seg_size(d); memcpy(e.gcm_hdr, d.stream_header, gcm::GCM_HEADER_LEN); }
         if (d.compression != PNA_COMPRESSION_NO) { e.seg_begin = (uint32_t)nsegs_total; e.n_segs = (uint32_t)enc_nsegs(d.plain.len); nsegs_total += e.n_segs; }
-        if (d.encryption) {
-            std::array<uint8_t, 33> k;
-            k[0] = d.encryption;
-            memcpy(k.data() + 1, d.key, 32);
-            auto it = key_ids.find(k);
-            if (it == key_ids.end()) {
-                DevKeys dk;
-                memset(&dk, 0, sizeof dk);
-                if (d.encryption == 1) {
-                    AesKey ak; aes256_expand_key(&ctx->h_aes, d.key, &ak);
-                    memcpy(dk.aes_rk, ak.rk, sizeof ak.rk); memcpy(dk.aes_dk, ak.dk, sizeof ak.dk);
-                } else {
-                    CamelliaKey ck; camellia256_expand_key(&ctx->h_cam, d.key, &ck);
-                    memcpy(dk.cam_ek, ck.ek, sizeof ck.ek); memcpy(dk.cam_dk, ck.dk, sizeof ck.dk);
-                }
-                it = key_ids.emplace(k, (int)E->h_keys.size()).first;
-                E->h_keys.push_back(dk);
-            }
-            e.key_idx = it->second;
-        }
+        if (d.encryption) e.key_idx = E->h_keys.index(ctx, d.encryption, d.key);
     }
     if (nsegs_total > 0xFFFFFFF0ull) return PNA_E_OOM;
     const uint64_t lit_base = align_up(plain_total, 256);
@@ -230,7 +204,7 @@ static int encode_plan_build(pna_ctx* ctx, const pna_encode_desc* descs, uint32_
     CK(E->d_work.reserve(E->work_bytes)); CK(E->d_out.reserve(E->out_bytes + 256));
     CK(E->d_entries.reserve(n)); CK(E->d_entries_init.reserve(n));
     CK(E->d_segs.reserve(nsegs_total)); CK(E->d_seqs.reserve(E->seq_total + 8)); CK(E->d_pieces.reserve(piece_cur + 1));
-    CK(E->d_keys.reserve(E->h_keys.size()));
+    CK(E->d_keys.reserve(E->h_keys.keys.size()));
     {
         // Upload of the plaintext.  A cudaMemcpyAsync costs the host 5-10 us whatever its size, which is what a group of
         // thousands of small files is made of -- so runs of entries whose host spans are exactly adjacent (files packed into one
@@ -276,7 +250,7 @@ static int encode_plan_build(pna_ctx* ctx, const pna_encode_desc* descs, uint32_
         }
     }
     cudaStream_t s = ctx->stream;
-    CK(E->d_entries_init.upload(E->h_entries, s)); CK(E->d_segs.upload(E->h_segs, s)); CK(E->d_keys.upload(E->h_keys, s));
+    CK(E->d_entries_init.upload(E->h_entries, s)); CK(E->d_segs.upload(E->h_segs, s)); CK(E->d_keys.upload(E->h_keys.keys, s));
     static enc::EncTables h_tables;
     static std::once_flag h_tables_once;   // plans are built concurrently by the host layer's worker threads
     std::call_once(h_tables_once, []() { enc::make_enc_tables(&h_tables); });
